@@ -3,6 +3,7 @@
 bench.py - fold matrices / second of the cvmatrix hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2|cfg3|cfg4|cfg5s] [--impl native|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the batched fold path (cvmx_training_batch: weight masses, numpy-order
 moments, DMMA Gram downdate, fused centering/scaling epilogue) over ALL folds of the workload, inputs
@@ -14,7 +15,8 @@ unmodified package staged in oracle/_ref by `make -C oracle ref` (kind "referenc
 restatement oracle/cvmatrix_oracle.py (kind "port") - on the box's host cores, all BLAS threads.
 `parity` compares the timed path's results with that reference on the same inputs (relative Frobenius error
 of XTX, XTY and the joint [XTX | XTY]; statistics bit for bit), `also` carries device-timed lines of the other
-two single-GPU workloads (cfg3, cfg4) measured in the same process.
+two single-GPU workloads (cfg3, cfg4) measured in the same process.  `--dump-outputs DIR` writes the results of the
+last timed step to DIR/<name>.npy (see dump_outputs), so that two builds can be compared output for output.
 
 Workloads (BASELINE.json configs; inputs per benchmarks/benchmark.py:223-232, seed 42, uniform [0,1)):
   cfg2  N=1,000,000 K=500 M=10 float64 weighted center+scale, 5 folds      (default; metric config)
@@ -75,7 +77,7 @@ CONFIGS = {
 }
 METRIC = "fold matrices/sec"
 UNIT = "fold-matrices/s"
-REF_BUDGET_S = 150.0   # wall-clock budget of the reference arm's warm-up + timed steps
+REF_BUDGET_S = 150.0   # wall-clock budget that bounds the reference arm's warm-up steps
 
 
 def fp64_peak_tflops():
@@ -217,8 +219,8 @@ def parity_summary(entries, kind, what):
 
 def run_reference(args, cfg, rank, world):
     """Reference arm: the reference's own CPU implementation at FULL size, all host threads; one step =
-    Partitioner + fit + every fold (training_XTX_XTY), exactly what benchmarks/benchmark.py:52-158 times.  The
-    number of timed steps is clamped so that warm-up + steps fit REF_BUDGET_S; the clamped numbers are printed."""
+    Partitioner + fit + every fold (training_XTX_XTY), exactly what benchmarks/benchmark.py:52-158 times.  Exactly
+    --steps steps are timed; warm-up steps after the first run only while they fit REF_BUDGET_S (their count is printed)."""
     if rank != 0:
         return
     RefCV, RefPart, kind, threads, blas = load_reference()
@@ -256,8 +258,7 @@ def run_reference(args, cfg, rank, world):
     while warmup < args.warmup and (time.perf_counter() - t_begin) + est * 2 < REF_BUDGET_S * 0.4:
         one_step()
         warmup += 1
-    left = REF_BUDGET_S - (time.perf_counter() - t_begin)
-    steps = int(max(1, min(args.steps, left // est)))
+    steps = args.steps
     t_fit = t_fold = 0.0
     for _ in range(steps):
         a, b = one_step()
@@ -301,6 +302,43 @@ def alloc_outputs(ctx, n, K, M):
     return dict(XTX=t.empty((n, K, K), dtype=t.float64, device=ctx.dev), XTY=t.empty((n, K, M), dtype=t.float64, device=ctx.dev),
                 stats=t.empty((n, 2, K + M), dtype=t.float64, device=ctx.dev), scal=t.empty((n, 2), dtype=t.float64, device=ctx.dev),
                 status=t.empty((n,), dtype=t.int32, device=ctx.dev))
+
+
+DUMP_LIMIT_BYTES = 60_000_000   # keeps a dump, .npy headers included, under 64 MB
+
+
+def dump_outputs(dirname, outs, first, n, K):
+    """Writes the results the timed step left in `outs` (n folds, CSR fold numbers first, first + 1, ...) as
+    dirname/<name>.npy: the arrays CVMatrix.training_batch returns, in the step's float dtype (status as float64),
+    plus `folds` and `rows`, the CSR fold numbers and the XTX / XTY rows written (float64).  Where the n folds exceed
+    DUMP_LIMIT_BYTES, a fixed seeded sample of them is written, and where one fold alone does, a fixed seeded sample
+    of the rows of its XTX and XTY.  A step of more folds than one output window holds (leave-one-out: 4096 folds
+    per chunk) leaves only its last chunk in `outs`, so the sample is drawn from that chunk."""
+    import torch
+
+    M = outs["XTY"].shape[2]
+    item = outs["XTX"].element_size()
+    per_fold = item * (K * K + K * M + 2 * (K + M) + 3)
+    rng = np.random.default_rng(0)
+    folds = np.arange(n)
+    if n * per_fold > DUMP_LIMIT_BYTES:
+        folds = np.sort(rng.choice(n, max(1, DUMP_LIMIT_BYTES // per_fold), replace=False))
+    rows = np.arange(K)
+    if per_fold > DUMP_LIMIT_BYTES:
+        rows = np.sort(rng.choice(K, DUMP_LIMIT_BYTES // (2 * item * (K + M)), replace=False))
+    dev = outs["XTX"].device
+    fi, ri = torch.from_numpy(folds).to(dev), torch.from_numpy(rows).to(dev)
+    pick = lambda name: outs[name].index_select(0, fi).cpu().numpy()  # noqa: E731
+    mats = {name: outs[name].index_select(0, fi).index_select(1, ri).cpu().numpy() for name in ("XTX", "XTY")}
+    stats, scal = pick("stats"), pick("scal")
+    arrays = dict(mats, X_mean=stats[:, 0:1, :K], X_std=stats[:, 1:2, :K], Y_mean=stats[:, 0:1, K:], Y_std=stats[:, 1:2, K:],
+                  sum_w_train=scal[:, 0], nnz_train=scal[:, 1], status=pick("status").astype(np.float64),
+                  folds=(folds + first).astype(np.float64), rows=rows.astype(np.float64))
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a))
+    print(f"bench.py: wrote {dirname}: {folds.size} of the {n} folds {first}..{first + n - 1}, {rows.size} of {K} rows of XTX "
+          f"and XTY", file=sys.stderr)
 
 
 def time_fold_path(ctx, m, P, steps, warmup, sf=None, row_sharded=False, clocks=False):
@@ -358,7 +396,8 @@ def time_fold_path(ctx, m, P, steps, warmup, sf=None, row_sharded=False, clocks=
         ctx.dist.all_reduce(t, op=ctx.dist.ReduceOp.MAX)
         ms = float(t.item())
     return dict(ms_per_step=ms / steps, prof_ms=[v / steps for v in prof_ms], prof_n=[v / steps for v in prof_n],
-                launches=int(launches), clocks=clk, outs=outs, fold_range=(f0, f1), chunk=chunk)
+                launches=int(launches), clocks=clk, outs=outs, fold_range=(f0, f1), chunk=chunk,
+                last_chunk=f0 + (f1 - f0 - 1) // chunk * chunk)   # first fold of the chunk the last step left in outs
 
 
 def roofline_of(cfg_name, cfg, world, rank_rows, rank_folds, timing, ms_per_step):
@@ -416,7 +455,7 @@ def run_row_slabs(args, cfg, ctx):
     f32 = bool(cfg.get("f32"))
     npdt, tdt = (np.float32, torch.float32) if f32 else (np.float64, torch.float64)
     B = 65536
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     warmup = 1
 
     gw = torch.Generator(device=dev)
@@ -490,6 +529,8 @@ def run_row_slabs(args, cfg, ctx):
     prof_ms, prof_n = (C.c_double * 3)(), (C.c_int64 * 3)()
     _lib.check(lib.cvmx_profile_read(h, prof_ms, prof_n), h)
     _lib.check(lib.cvmx_profile_enable(h, 0), h)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs, o0, o1 - o0, K)
     # end to end: fit from the device-generated blocks + all folds + every result copied to pinned host memory
     host_out = {k: torch.empty(v.shape, dtype=v.dtype, pin_memory=True) for k, v in outs.items() if v is not None}
     ctx.barrier()
@@ -573,11 +614,18 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the comparison with the CPU reference (N > 1: one fold on rank 0)")
     ap.add_argument("--e2e-out", default="numpy", choices=["numpy", "pinned"],
                     help="host destination of the e2e results: fresh numpy arrays (the reference's convention) or the reused page-locked pool")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (above 64 MB, or beyond one output window of "
+                         "4096 folds: a fixed, seeded sample of the last window)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
+    if args.dump_outputs and (args.impl != "native" or world > 1 or os.environ.get("BENCH_EMULATE_SHARDS", "0") != "0"):
+        ap.error("--dump-outputs writes the native path's results of a single process (--impl native, one rank, no shard emulation)")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
 
     if args.impl == "reference":
@@ -643,6 +691,8 @@ def main():
         rank_rows, rank_folds = int(part.offsets[f1] - part.offsets[f0]), f1 - f0
     roof = roofline_of(args.config, cfg, world, rank_rows, rank_folds, tm, ms_per_step)
     outs, clocks, launches = tm["outs"], tm["clocks"], tm["launches"]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs, tm["last_chunk"], f1 - tm["last_chunk"], K)
 
     # results of the timed path for the parity block (before e2e refits the handle)
     want_parity = not args.no_parity and not emulate
@@ -665,7 +715,7 @@ def main():
         else:
             torch.cuda.synchronize()
             if rank == 0:     # first fold of rank 0's own block
-                lo = f0 + ((f1 - f0 - 1) // tm["chunk"]) * tm["chunk"]   # the chunk that is still in the output window
+                lo = tm["last_chunk"]   # the chunk that is still in the output window
                 st = outs["stats"][0].cpu().numpy()
                 native_res[lo] = (outs["XTX"][0].cpu().numpy(), outs["XTY"][0].cpu().numpy(), (st[0, :K], st[1, :K], st[0, K:], st[1, K:]))
 
@@ -673,7 +723,7 @@ def main():
     also = None
     if args.config == "cfg2" and not args.no_also and not emulate:
         also = {}
-        a_steps, a_warm = max(3, min(args.steps, 8)), 3
+        a_steps, a_warm = args.steps, args.warmup
         c3 = CONFIGS["cfg3"]
         m.set_folds(Partitioner(np.arange(N) % c3["P"]))
         t3 = time_fold_path(ctx, m, c3["P"], a_steps, a_warm)
@@ -704,7 +754,7 @@ def main():
     if not args.no_e2e:
         if world == 1:
             _lib.check(lib.cvmx_set_stream(h, None), h)
-        e2e_steps = args.steps if cfg["P"] <= 1000 else max(1, min(args.steps, 2))
+        e2e_steps = args.steps
         out_bytes = 0
         host_out = None
         fb0, fb1 = rank * P // world, (rank + 1) * P // world
@@ -804,11 +854,11 @@ def main():
             Xp, Yp, wp = np.array(X), np.array(Y), np.array(w)
             e2e_step(Xp, Yp, wp)
             t0 = time.perf_counter()
-            for _ in range(2):
+            for _ in range(args.steps):
                 e2e_step(Xp, Yp, wp)
             torch.cuda.synchronize()
-            dtp = (time.perf_counter() - t0) / 2
-            e2e["pageable_input"] = {"value": P / dtp, "unit": UNIT, "ms_per_step": dtp * 1e3, "steps": 2,
+            dtp = (time.perf_counter() - t0) / args.steps
+            e2e["pageable_input"] = {"value": P / dtp, "unit": UNIT, "ms_per_step": dtp * 1e3, "steps": args.steps,
                                      "note": "inputs are ordinary (pageable) numpy arrays: the library stages them through its page-locked ring filled by worker threads "
                                              "(csrc/host_stager.h; CVMX_HOST_STAGER=0 = the driver's bounce buffer, ~370 ms)"}
             del Xp, Yp, wp

@@ -1,7 +1,7 @@
 """
 CPU tests (-m "not gpu"): the two oracles (numpy port in both summation orders, plain-C
-restatement) against the golden fixtures frozen from the live reference, plus a live
-re-check when /root/reference is present.
+restatement) against the golden fixtures frozen from the live reference, the pinning grid of
+oracle/check_against_reference.py from its stored outputs, and that grid live where the reference is staged.
 
 Tolerances: statistics, weight sums, Partitioner outputs and error strings are compared
 bit-exactly.  Matrices from the numpy port are compared at relFro <= 1e-14 (f64) because
@@ -16,12 +16,14 @@ import sys
 import numpy as np
 import pytest
 
+import check_against_reference
 import golden_io
 from cvmatrix_oracle import OracleCVMatrix, OraclePartitioner, pairwise_sum, rel_fro, sequential_colsum
 import c_oracle
 
 STATS = ("X_mean", "X_std", "Y_mean", "Y_std")
 TOL = {"float64": 1e-12, "float32": 1e-5}
+PIN_GRID = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "pin_grid.npz")
 
 
 def _unpack(method, res):
@@ -137,7 +139,20 @@ def test_summation_orders_match_numpy():
         assert np.array_equal(c_oracle.colsum(A), np.sum(A, axis=0, keepdims=True))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="live reference only exists in the build container")
+def test_oracle_matches_pinned_grid():
+    """The pinning grid of oracle/check_against_reference.py, offline (tests/golden/pin_grid.npz): Partitioner outputs,
+    statistics, weight sums and error messages bit for bit; matrices, whose bits depend on the host's BLAS, to
+    relFro <= 1e-14 (float64) / 1e-6 (float32); both summation orders."""
+    want, _ = check_against_reference.load_recorded(PIN_GRID)
+    assert len(want) > 30_000
+    for order in ("numpy", "explicit"):
+        bad = check_against_reference.compare(check_against_reference.grid_outputs(*check_against_reference.oracle_classes(order)),
+                                              want, matrix_tol=1e-14)
+        assert not bad, (order, len(bad), bad[:10])
+
+
+@pytest.mark.skipif(not os.path.isfile(os.path.join(check_against_reference.REF, "cvmatrix", "cvmatrix.py")),
+                    reason="needs the unmodified reference: oracle/_ref staged by `make -C oracle ref`, or CVMATRIX_REFERENCE")
 def test_oracle_pinned_to_live_reference():
     script = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "check_against_reference.py")
     r = subprocess.run([sys.executable, script], capture_output=True, text=True)
