@@ -52,6 +52,7 @@ SIGNATURES = {
     "cvmx_slab_fold_sums": (_i32, [_vp, _i64, _i64, _vp]),
     "cvmx_slab_finalize_stats": (_i32, [_vp, _i64, _i64, _vp]),
     "cvmx_validation_rows": (_i32, [_vp, _i64, _vp, _u32, _vp, _vp, _i32]),
+    "cvmx_pls_cv": (_i32, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i32]),
     "cvmx_profile_enable": (_i32, [_vp, _i32]),
     "cvmx_profile_read": (_i32, [_vp, C.POINTER(_dbl), C.POINTER(_i64)]),
     "cvmx_partition_labels": (_i64, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp]),

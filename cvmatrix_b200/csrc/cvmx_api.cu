@@ -14,6 +14,7 @@
 #include "kernels_gram.cuh"
 #include "kernels_gram_tc.cuh"
 #include "kernels_scan.cuh"
+#include "kernels_pls.cuh"
 #include <cstdlib>
 #include <type_traits>
 
@@ -92,6 +93,8 @@ struct cvmx_handle {
   // reference), 1 exact form (numpy's operation order and IEEE division: bit-identical matrices for one-row folds)
   int loo_mode = 0;
   DevBuf loo_ops;
+  // cross-validated PLS (cvmx_pls_cv): per-window working state, PRESS chunk table and partials, staged host outputs
+  DevBuf pls_ws, pls_tab, pls_part, pls_out;
   // fused fit + folds (cvmx_fit_folds): raw float64 Gram of every fold of a true partition, [P][ntiles][GACC][GTHREADS],
   // valid while csr_version == fold_gram_version; cvmx_training_batch then only runs statistics + epilogue
   TableCache tc_gram, tc_finish;
@@ -1714,6 +1717,119 @@ int32_t training_impl(cvmx_t* h, const int64_t* d_off, const int64_t* d_idx, con
   return CVMX_OK;
 }
 
+// Cross-validated PLS over folds [f0, f1) (include/cvmx.h: cvmx_pls_cv).  The range is walked in windows that keep the
+// device scratch near 1 GiB, as training_impl stages host outputs: run_folds leaves the window's XTX / XTY, statistics and
+// fold scalars in library scratch, the PLS kernels fit every fold, the PRESS kernels score its validation rows.
+template <typename T>
+int32_t pls_cv_impl(cvmx_t* h, int64_t f0, int64_t f1, int64_t A, void* opress, void* osumw, void* oB, int32_t* onfit,
+                    int32_t* ostatus, int32_t mem) {
+  const size_t sz = sizeof(T);
+  const int64_t K = h->K, M = h->M;
+  const uint32_t want = CVMX_WANT_XTX | CVMX_WANT_XTY;
+  const bool host = mem == CVMX_HOST;
+  const size_t ws_fold = pls_state_doubles(K, M, A) * sizeof(double) + 2 * sizeof(int32_t);
+  const size_t out_fold = host ? (size_t)A * M * sz + sz + 2 * sizeof(int32_t) + (oB ? (size_t)A * K * M * sz : 0) : 0;
+  const size_t per_fold = (size_t)(K * K + K * M) * sz + ws_fold + out_fold;
+  const int64_t chunk = std::max<int64_t>(1, (int64_t)(((size_t)1 << 30) / per_fold));
+  const cudaMemcpyKind kind = host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  const size_t smem_dir = M > 1 ? (size_t)(M * M + PLS_CH * M) * sizeof(double) : 0;
+  const size_t smem_press = press_smem_bytes(M);
+  CU(h, cudaFuncSetAttribute(k_pls_dir, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_dir));
+  CU(h, cudaFuncSetAttribute(k_pls_press<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_press));
+  const int64_t* off = h->h_off.data();
+  std::vector<int64_t> tab;
+  for (int64_t c0 = f0; c0 < f1; c0 += chunk) {
+    const int64_t c1 = std::min(f1, c0 + chunk), Pn = c1 - c0, d = c0 - f0;
+    CU(h, h->out_xx.reserve((size_t)Pn * K * K * sz));
+    CU(h, h->out_xy.reserve((size_t)Pn * K * M * sz));
+    int32_t rc = run_folds<T>(h, h->d_off.as<int64_t>(), h->d_idx.as<int64_t>(), off, c0, c1, want, h->out_xx.as<T>(),
+                              h->out_xy.as<T>(), chunk >= f1 - f0);
+    if (rc) return rc;
+    // working state
+    CU(h, h->pls_ws.reserve((size_t)Pn * ws_fold));
+    PlsState st;
+    st.K = K; st.M = M; st.A = A;
+    double* q = h->pls_ws.as<double>();
+    st.xty = q; q += Pn * K * M;
+    st.R = q; q += Pn * A * K;
+    st.Pm = q; q += Pn * A * K;
+    st.Q = q; q += Pn * A * M;
+    st.u = q; q += Pn * K;
+    st.S = q; q += Pn * 2 * M * M;
+    st.y0 = q; q += Pn;
+    st.nfit = reinterpret_cast<int32_t*>(q);
+    st.state = st.nfit + Pn;
+    k_pls_init<T><<<(unsigned)Pn, PLS_THREADS, 0, h->stream>>>(h->out_xy.as<T>(), h->fscal.as<FoldScalars>(), h->flags, st);
+    h->launches++;
+    const dim3 gxr((unsigned)Pn, (unsigned)((K + PLS_ROWS_PER_BLOCK - 1) / PLS_ROWS_PER_BLOCK));
+    for (int64_t a = 0; a < A; ++a) {
+      k_pls_dir<<<(unsigned)Pn, PLS_THREADS, smem_dir, h->stream>>>(st, a);
+      k_pls_xtx_r<T><<<gxr, PLS_THREADS, 0, h->stream>>>(h->out_xx.as<T>(), st, a);
+      k_pls_update<<<(unsigned)Pn, PLS_THREADS, 0, h->stream>>>(st, a);
+      h->launches += 3;
+    }
+    CU(h, cudaGetLastError());
+    // PRESS: chunks of at most PRESS_ROWS validation rows, never spanning two folds; then chunk_off [Pn + 1]
+    tab.clear();
+    std::vector<int64_t> coff((size_t)Pn + 1, 0);
+    for (int64_t f = c0; f < c1; ++f) {
+      for (int64_t p = off[f]; p < off[f + 1]; p += PRESS_ROWS) {
+        tab.push_back(p);
+        tab.push_back(std::min<int64_t>(PRESS_ROWS, off[f + 1] - p));
+        tab.push_back(f - c0);
+      }
+      coff[f - c0 + 1] = (int64_t)tab.size() / 3;
+    }
+    const int64_t nch = (int64_t)tab.size() / 3;
+    tab.insert(tab.end(), coff.begin(), coff.end());
+    CU(h, h->pls_tab.reserve(tab.size() * sizeof(int64_t)));
+    CU(h, cudaMemcpyAsync(h->pls_tab.p, tab.data(), tab.size() * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
+    CU(h, h->pls_part.reserve((size_t)std::max<int64_t>(nch, 1) * (A * M + 1) * sizeof(double)));
+    double* part = h->pls_part.as<double>();
+    double* part_w = part + nch * A * M;
+    if (nch > 0) {
+      PressParams<T> pp;
+      pp.Z = h->Z.as<T>(); pp.w = h->weighted ? h->w.as<T>() : nullptr; pp.ld = h->ld;
+      pp.idx = h->d_idx.as<int64_t>(); pp.chunks = h->pls_tab.as<int64_t>(); pp.stats = h->stats.as<T>();
+      pp.flags = h->flags; pp.s = st; pp.part = part; pp.part_w = part_w;
+      k_pls_press<T><<<(unsigned)nch, PLS_THREADS, smem_press, h->stream>>>(pp);
+      h->launches++;
+    }
+    // outputs: straight into the caller's device buffers, or staged for the copy to the host
+    T *dpress = (T*)opress + (size_t)d * A * M, *dsumw = (T*)osumw + d, *dB = oB ? (T*)oB + (size_t)d * A * K * M : nullptr;
+    int32_t* dstatus = ostatus + d;
+    if (host) {
+      CU(h, h->pls_out.reserve((size_t)Pn * out_fold));
+      char* o = h->pls_out.as<char>();
+      dpress = (T*)o; o += (size_t)Pn * A * M * sz;
+      dsumw = (T*)o; o += (size_t)Pn * sz;
+      dstatus = (int32_t*)o; o += (size_t)Pn * sizeof(int32_t);
+      o += (size_t)Pn * sizeof(int32_t);
+      dB = oB ? (T*)o : nullptr;
+    }
+    k_pls_press_reduce<T><<<(unsigned)Pn, PLS_THREADS, 0, h->stream>>>(part, part_w, h->pls_tab.as<int64_t>() + 3 * nch, st,
+                                                                       dpress, dsumw);
+    k_pack_scalars<T><<<(unsigned)((Pn + 255) / 256), 256, 0, h->stream>>>(h->fscal.as<FoldScalars>(), Pn, nullptr, dstatus);
+    h->launches += 2;
+    if (dB) {
+      const dim3 gc((unsigned)Pn, (unsigned)std::min<int64_t>(65535, (K * M + PLS_THREADS - 1) / PLS_THREADS));
+      k_pls_coefs<T><<<gc, PLS_THREADS, 0, h->stream>>>(st, dB);
+      h->launches++;
+    }
+    CU(h, cudaGetLastError());
+    CU(h, cudaMemcpyAsync(onfit + d, st.nfit, (size_t)Pn * sizeof(int32_t), kind, h->stream));
+    if (host) {
+      CU(h, cudaMemcpyAsync((char*)opress + (size_t)d * A * M * sz, dpress, (size_t)Pn * A * M * sz, kind, h->stream));
+      CU(h, cudaMemcpyAsync((T*)osumw + d, dsumw, (size_t)Pn * sz, kind, h->stream));
+      CU(h, cudaMemcpyAsync(ostatus + d, dstatus, (size_t)Pn * sizeof(int32_t), kind, h->stream));
+      if (oB) CU(h, cudaMemcpyAsync((char*)oB + (size_t)d * A * K * M * sz, dB, (size_t)Pn * A * K * M * sz, kind, h->stream));
+    }
+    // the next window reuses the scratch and the chunk table's host vector
+    CU(h, cudaStreamSynchronize(h->stream));
+  }
+  return CVMX_OK;
+}
+
 // offsets: always a host array here; indices: host or device according to `mem`
 int32_t upload_csr(cvmx_t* h, DevBuf& doff, DevBuf& didx, const int64_t* offsets, const int64_t* indices, int64_t P,
                    int64_t nidx, int32_t mem) {
@@ -1831,7 +1947,8 @@ int32_t cvmx_destroy(cvmx_t* h) {
   cudaStreamSynchronize(h->stream);
   for (DevBuf* b : {&h->stat_flags, &h->peer_sum, &h->w_glob, &h->g_off, &h->g_idx, &h->scan_look, &h->loo_ops, &h->Z, &h->w, &h->Ttot, &h->sum_z, &h->sumsq_z, &h->fit_scal, &h->d_off, &h->d_idx, &h->a_off, &h->a_idx,
                     &h->units, &h->tiles, &h->fold_units, &h->split_folds, &h->partials, &h->stats, &h->rawsums, &h->fscal, &h->pwcols,
-                    &h->errflag, &h->out_xx, &h->out_xy, &h->out_small, &h->scan_seg, &h->scan_ok, &h->scan_list, &h->scan_cnt, &h->ystage, &h->fold_gram, &h->fold_raw, &h->chunk_ranges})
+                    &h->errflag, &h->out_xx, &h->out_xy, &h->out_small, &h->scan_seg, &h->scan_ok, &h->scan_list, &h->scan_cnt, &h->ystage, &h->fold_gram, &h->fold_raw, &h->chunk_ranges,
+                    &h->pls_ws, &h->pls_tab, &h->pls_part, &h->pls_out})
     b->release();
   h->tc_gram.release(); h->tc_finish.release();
   delete h->stager; h->stager = nullptr;
@@ -2266,6 +2383,24 @@ int32_t cvmx_validation_rows(cvmx_t* h, int64_t fold, const void* stats, uint32_
   ON_DEVICE(h);
   return h->dtype == CVMX_F64 ? validation_rows_impl<double>(h, fold, stats, apply, out_X, out_Y, mem)
                               : validation_rows_impl<float>(h, fold, stats, apply, out_X, out_Y, mem);
+}
+
+int32_t cvmx_pls_cv(cvmx_t* h, int64_t f0, int64_t f1, int64_t n_components, void* out_press, void* out_sum_w_val, void* out_B,
+                    int32_t* out_n_fitted, int32_t* out_status, int32_t mem) {
+  if (!h || !h->fitted) return fail(h, CVMX_ERR_INVALID, "cvmx_pls_cv: fit first");
+  if (h->slab) return fail(h, CVMX_ERR_INVALID, "cvmx_pls_cv: not available for a row-slab handle");
+  if (f0 < 0 || f1 > h->P || f0 > f1) return fail(h, CVMX_ERR_INVALID, "cvmx_pls_cv: fold range outside the CSR");
+  if (h->M == 0) return fail(h, CVMX_ERR_NO_Y, "Response variables `Y` are not provided.");
+  if (n_components < 1 || n_components > h->K)
+    return fail(h, CVMX_ERR_INVALID, "n_components must be between 1 and the number of columns of X (" + std::to_string(h->K) + ")");
+  if (h->M > PLS_MAX_M)
+    return fail(h, CVMX_ERR_INVALID, "cvmx_pls_cv: at most " + std::to_string(PLS_MAX_M) + " response columns are supported");
+  if (f1 > f0 && (!out_press || !out_sum_w_val || !out_n_fitted || !out_status))
+    return fail(h, CVMX_ERR_INVALID, "cvmx_pls_cv: an output pointer is NULL");
+  ON_DEVICE(h);
+  return h->dtype == CVMX_F64
+             ? pls_cv_impl<double>(h, f0, f1, n_components, out_press, out_sum_w_val, out_B, out_n_fitted, out_status, mem)
+             : pls_cv_impl<float>(h, f0, f1, n_components, out_press, out_sum_w_val, out_B, out_n_fitted, out_status, mem);
 }
 
 int32_t cvmx_profile_enable(cvmx_t* h, int32_t on) {

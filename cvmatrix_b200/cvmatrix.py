@@ -18,7 +18,9 @@ exceptions (cvmatrix/cvmatrix.py:625-629, 1074-1078).
 
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
+import warnings
 from typing import Optional, Sequence, Tuple, Union
 
 import numpy as np
@@ -38,6 +40,10 @@ _ERR_NO_Y = "Response variables `Y` are not provided."
 
 def _ptr(a: Optional[np.ndarray]):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def _tptr(t):
+    return None if t is None else C.c_void_p(t.data_ptr())
 
 
 class CVMatrix:
@@ -472,7 +478,6 @@ class CVMatrix:
         want = (_lib.WANT_XTX if return_XTX else 0) | (_lib.WANT_XTY if return_XTY else 0)
         cX, cY, sX, sY = self.center_X, self.center_Y, self.scale_X, self.scale_Y
         need = (cX or (return_XTY and cY), sX, return_XTY and (cX or cY), return_XTY and sY)
-        bound, prev_stream = False, None
         if out == "torch":
             import torch
 
@@ -483,16 +488,8 @@ class CVMatrix:
             stats = torch.empty((P, 2, K + M), dtype=tdt, device=dev)
             scal = torch.empty((P, 2), dtype=tdt, device=dev)
             status = torch.empty((P,), dtype=torch.int32, device=dev)
-            p = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
+            p = _tptr
             mem = _lib.DEVICE
-            # run stream-ordered with torch so the freshly allocated outputs are safe to write; the legacy
-            # default stream has no handle to share, so order against it with a full synchronisation instead
-            ts = torch.cuda.current_stream(dev)
-            if ts.cuda_stream:
-                _lib.check(self._lib.cvmx_set_stream(self._h, C.c_void_p(ts.cuda_stream)), self._h)
-                bound = True
-            else:
-                ts.synchronize()
         elif out == "pinned":
             # page-locked host arrays from a pool that is REUSED by the next out="pinned" call: the device->host copy
             # then runs at the PCIe rate (a copy into fresh pageable numpy memory is bounded by page faults and the
@@ -514,15 +511,9 @@ class CVMatrix:
             mem = _lib.HOST
         else:
             raise ValueError("out must be 'numpy', 'pinned' or 'torch'")
-        try:
+        with self._torch_stream() if out == "torch" else contextlib.nullcontext():
             rc = self._lib.cvmx_training_batch(self._h, fold_begin, fold_end, want, p(XTX), p(XTY), p(stats), p(scal), p(status), mem)
             _lib.check(rc, self._h)
-        finally:
-            if out == "torch":
-                if bound:   # always unbind: a failed call must not leave the handle on the caller's stream
-                    self._lib.cvmx_set_stream(self._h, prev_stream)  # syncs, back to the private stream
-                else:       # legacy default stream: the results must be complete before torch touches them
-                    self._lib.cvmx_sync(self._h)
         if check:
             st = status.cpu().numpy() if out == "torch" else status
             for s in np.unique(st):
@@ -535,6 +526,103 @@ class CVMatrix:
             Y_mean=mean[:, :, K:] if need[2] else None, Y_std=std[:, :, K:] if need[3] else None,
             sum_w_train=scal[:, 0], nnz_train=scal[:, 1], status=status,
         )
+
+    @contextlib.contextmanager
+    def _torch_stream(self):
+        """Runs the enclosed library calls stream-ordered with torch's current stream, so that freshly allocated torch
+        outputs are safe to write.  The legacy default stream has no handle to share: the library then orders against it
+        with a full synchronisation instead."""
+        import torch
+
+        ts = torch.cuda.current_stream(torch.device("cuda", self.device))
+        bound = False
+        if ts.cuda_stream:
+            _lib.check(self._lib.cvmx_set_stream(self._h, C.c_void_p(ts.cuda_stream)), self._h)
+            bound = True
+        else:
+            ts.synchronize()
+        try:
+            yield
+        finally:
+            if bound:   # always unbind: a failed call must not leave the handle on the caller's stream
+                self._lib.cvmx_set_stream(self._h, None)  # syncs, back to the private stream
+            else:       # legacy default stream: the results must be complete before torch touches them
+                self._lib.cvmx_sync(self._h)
+
+    def pls_cross_validate(self, n_components: int, fold_begin: int = 0, fold_end: Optional[int] = None,
+                           return_coefs: bool = False, out: str = "numpy", check: bool = True):
+        """
+        Cross-validated PLS regression over folds ``[fold_begin, fold_end)`` of the CSR (see ``set_folds``), on the GPU.
+
+        Every fold's model is fitted by Improved Kernel PLS (Algorithm 2 of Dayal & MacGregor, 1997) in float64 from
+        the fold's ``XTX`` / ``XTY`` and training statistics exactly as ``training_batch`` forms them, for
+        ``n_components`` = A components.  The fold's validation rows are then predicted with 1 .. A components,
+        ``((x - X_mean) / X_std) @ B * Y_std + Y_mean`` (each statistic applied iff its flag is set), and scored.
+
+        Returns a dict with ``press`` (P, A, M): the weighted sum of squared prediction errors over the validation rows,
+        ``sum_w_val`` (P,): the sum of their weights (their count when unweighted), ``n_fitted`` (P,) int32: the
+        components a fold could fit (a fold whose remaining ``XTY`` vanishes stops early; its later coefficients repeat
+        the last ones), ``status`` (P,) int32 (``CVMX_FOLD_*`` bits) and ``B`` (P, A, K, M) with ``return_coefs``,
+        else None.  ``out="torch"`` returns CUDA tensors, ``out="numpy"`` host arrays.  With ``check`` the degenerate fold
+        errors of ``training_XTX_XTY`` are raised; without it such folds get NaN ``press`` / ``B`` and ``n_fitted`` 0.
+        A ``UserWarning`` names folds that stopped early.
+
+        Example - root mean squared error of cross-validation per number of components and response::
+
+            cvm.fit(X, Y); cvm.set_folds(Partitioner(folds))
+            r = cvm.pls_cross_validate(20)
+            rmsecv = np.sqrt(r["press"].sum(0) / r["sum_w_val"].sum())    # (20, M)
+        """
+        self._require_fit()
+        if fold_end is None:
+            fold_end = self._n_folds
+        if not self._has_Y:
+            raise ValueError(_ERR_NO_Y)
+        A, K, M, dt = int(n_components), self.K, self.M, self.dtype
+        if not 1 <= A <= K:
+            raise ValueError(f"n_components must be between 1 and the number of columns of X ({K}); got {A}")
+        if M > 128:
+            raise ValueError(f"at most 128 response columns are supported; Y has {M}")
+        P = max(int(fold_end) - int(fold_begin), 0)
+        if out == "torch":
+            import torch
+
+            tdt = torch.float64 if np.dtype(dt) == np.float64 else torch.float32
+            dev = torch.device("cuda", self.device)
+            press = torch.empty((P, A, M), dtype=tdt, device=dev)
+            sum_w = torch.empty((P,), dtype=tdt, device=dev)
+            n_fitted = torch.empty((P,), dtype=torch.int32, device=dev)
+            status = torch.empty((P,), dtype=torch.int32, device=dev)
+            B = torch.empty((P, A, K, M), dtype=tdt, device=dev) if return_coefs else None
+            p, mem = _tptr, _lib.DEVICE
+        elif out == "numpy":
+            press = np.empty((P, A, M), dt)
+            sum_w = np.empty((P,), dt)
+            n_fitted = np.zeros((P,), np.int32)
+            status = np.zeros((P,), np.int32)
+            B = np.empty((P, A, K, M), dt) if return_coefs else None
+            p, mem = _ptr, _lib.HOST
+        else:
+            raise ValueError("out must be 'numpy' or 'torch'")
+        with self._torch_stream() if out == "torch" else contextlib.nullcontext():
+            rc = self._lib.cvmx_pls_cv(self._h, int(fold_begin), int(fold_end), A, p(press), p(sum_w), p(B), p(n_fitted),
+                                       p(status), mem)
+            _lib.check(rc, self._h)
+        st = status.cpu().numpy() if out == "torch" else status
+        if check:
+            cX, cY, sX, sY = self.center_X, self.center_Y, self.scale_X, self.scale_Y
+            need = (cX or cY, sX, cX or cY, sY)    # the statistics training_XTX_XTY computes
+            for s in np.unique(st):
+                if s:
+                    self._raise_for_status(int(s), need)
+        nf = n_fitted.cpu().numpy() if out == "torch" else n_fitted
+        refused = (((st & _lib.FOLD_NO_NONZERO_W) != 0) & (self._flags != 0)) | (((st & _lib.FOLD_NNZ_LE_DDOF) != 0) & ((self._flags & 12) != 0))
+        early = np.flatnonzero((nf < A) & ~refused)
+        if early.size:
+            warnings.warn(f"{early.size} fold(s) stopped before {A} components (first: fold {int(fold_begin) + int(early[0])} "
+                          f"with {int(nf[early[0]])}): the remaining XTY vanished; their later coefficients repeat the last ones",
+                          UserWarning, stacklevel=2)
+        return dict(press=press, sum_w_val=sum_w, n_fitted=n_fitted, status=status, B=B)
 
     def validation_rows(self, fold: int, stats: Optional[Stats] = None, out: str = "numpy"):
         """

@@ -270,6 +270,27 @@ int32_t cvmx_slab_finalize_stats(cvmx_t* h, int64_t f0, int64_t f1, const void* 
 int32_t cvmx_validation_rows(cvmx_t* h, int64_t fold, const void* stats, uint32_t apply, void* out_X, void* out_Y,
                              int32_t mem);
 
+/*
+ * Cross-validated PLS regression over folds [fold_begin, fold_end) of the CSR - the consumer of the training matrices
+ * (ikpls after training_XTX_XTY, cvmatrix/partitioner.py:27-31).  Per fold, from XTX / XTY and the statistics exactly as
+ * cvmx_training_batch(XTX | XTY) forms them: Improved Kernel PLS, Algorithm 2 (Dayal & MacGregor 1997) with A =
+ * n_components components in float64 (M > 1: the direction is the dominant eigenvector of XTY_a^T XTY_a; a fold stops
+ * early when ||XTY_a q|| <= 64 eps ||XTY_0||_F or t^T t <= 0, later coefficients repeat the last ones), then the
+ * validation rows x_i of the fold predict y^_i = ((x_i - mu_X) / sigma_X) B_a * sigma_Y + mu_Y (each statistic applied
+ * iff its flag is set) for a = 0 .. A-1.  With P' = fold_end - fold_begin, in the handle's dtype unless noted:
+ *   out_press      [P', A, M]     sum over the validation rows (as stored: repeats count) of w_i (y_im - y^_im)^2
+ *   out_sum_w_val  [P']           sum of the validation weights (row count when unweighted)
+ *   out_B          [P', A, K, M]  coefficients B_a (may be NULL)
+ *   out_n_fitted   [P'] int32     components fitted before the fold stopped (<= A)
+ *   out_status     [P'] int32     CVMX_FOLD_* bits
+ * Folds whose status bits make training_XTX_XTY raise (cvmatrix/cvmatrix.py:625-629, 1074-1078) get NaN press and B and
+ * n_fitted = 0.  The range is processed in windows of about 1 GiB of device scratch; a range that fits one window reuses
+ * the fold Grams kept by cvmx_fit_folds.  M = 0 gives CVMX_ERR_NO_Y; A outside [1, K] or M > 128 CVMX_ERR_INVALID.
+ * `mem` applies to all five outputs.  Results do not depend on the launch geometry: identical calls give identical bits.
+ */
+int32_t cvmx_pls_cv(cvmx_t* h, int64_t fold_begin, int64_t fold_end, int64_t n_components, void* out_press,
+                    void* out_sum_w_val, void* out_B, int32_t* out_n_fitted, int32_t* out_status, int32_t mem);
+
 /* Per-kernel device timing for bench.py's roofline line: while enabled, CUDA events are recorded on the
  * handle's stream around the statistics kernels (ms[0]), the Gram kernel (ms[1]) and the split-reduce
  * kernel (ms[2]); cvmx_profile_read synchronises, returns the accumulated milliseconds and span counts
