@@ -14,6 +14,19 @@ HOST, DEVICE = 0, 1
 WANT_XTX, WANT_XTY, WANT_STATS = 1, 2, 4
 FOLD_NO_NONZERO_W, FOLD_NNZ_LE_DDOF = 1, 2
 
+# cvmx_ridge_plan (include/cvmx.h): kernels (CVMX_RK_*) and plan entries (CVMX_RIDGE_*)
+(RK_LOAD, RK_POTRF, RK_TRSM, RK_SYRK, RK_BSOLVE_DIAG, RK_BSOLVE_UPDATE, RK_PRESS, RK_PRESS_ACCUM, RK_FINISH,
+ RK_COEFS) = range(10)
+RK_COUNT = 10
+RIDGE_KERNELS = ("k_ridge_load", "k_ridge_potrf_diag", "k_ridge_trsm", "k_ridge_syrk", "k_ridge_bsolve_diag",
+                 "k_ridge_bsolve_update", "k_ridge_press", "k_ridge_press_accum", "k_ridge_finish", "k_ridge_coefs")
+(RIDGE_FEASIBLE, RIDGE_FOLDS_PER_WINDOW, RIDGE_PENALTIES_PER_PASS, RIDGE_SCRATCH_BYTES, RIDGE_END_A, RIDGE_END_STATE,
+ RIDGE_END_ACC, RIDGE_END_ACC_W, RIDGE_END_PRESS, RIDGE_END_INFO, RIDGE_END_B, RIDGE_END_SUM_W, RIDGE_END_STATUS,
+ RIDGE_WINDOW_BYTES, RIDGE_PART_BYTES, RIDGE_CHUNKS_PER_LAUNCH) = range(16)
+RIDGE_GRID = 16
+RIDGE_SMEM = RIDGE_GRID + 2 * RK_COUNT
+RIDGE_PLAN_LEN = RIDGE_SMEM + RK_COUNT
+
 _vp, _i64, _i32, _u32, _dbl = C.c_void_p, C.c_int64, C.c_int32, C.c_uint32, C.c_double
 
 # name -> (restype, argtypes); mirrors include/cvmx.h one to one (tests check the export list)
@@ -53,6 +66,8 @@ SIGNATURES = {
     "cvmx_slab_finalize_stats": (_i32, [_vp, _i64, _i64, _vp]),
     "cvmx_validation_rows": (_i32, [_vp, _i64, _vp, _u32, _vp, _vp, _i32]),
     "cvmx_pls_cv": (_i32, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i32]),
+    "cvmx_ridge_cv": (_i32, [_vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _i32]),
+    "cvmx_ridge_plan": (_i32, [_i64, _i64, _i64, _i64, _i32, _i32, _i32, _vp]),
     "cvmx_profile_enable": (_i32, [_vp, _i32]),
     "cvmx_profile_read": (_i32, [_vp, C.POINTER(_dbl), C.POINTER(_i64)]),
     "cvmx_partition_labels": (_i64, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp]),

@@ -18,7 +18,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcvmx.so")
 SOURCES = ["cvmx_api.cu"]
-HEADERS = ["host_stager.h", "common.cuh", "kernels_stats.cuh", "kernels_scan.cuh", "kernels_gram.cuh", "kernels_gram_tc.cuh", "kernels_pls.cuh", os.path.join("..", "..", "include", "cvmx.h")]
+HEADERS = ["host_stager.h", "common.cuh", "kernels_stats.cuh", "kernels_scan.cuh", "kernels_gram.cuh", "kernels_gram_tc.cuh", "kernels_pls.cuh", "kernels_ridge.cuh", os.path.join("..", "..", "include", "cvmx.h")]
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

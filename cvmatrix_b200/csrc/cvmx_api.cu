@@ -15,6 +15,7 @@
 #include "kernels_gram_tc.cuh"
 #include "kernels_scan.cuh"
 #include "kernels_pls.cuh"
+#include "kernels_ridge.cuh"
 #include <cstdlib>
 #include <type_traits>
 
@@ -95,6 +96,8 @@ struct cvmx_handle {
   DevBuf loo_ops;
   // cross-validated PLS (cvmx_pls_cv): per-window working state, PRESS chunk table and partials, staged host outputs
   DevBuf pls_ws, pls_tab, pls_part, pls_out;
+  // cross-validated ridge (cvmx_ridge_cv): pass scratch (cvmx_ridge_plan's layout), PRESS chunk table and partials, penalties
+  DevBuf ridge_ws, ridge_tab, ridge_part, ridge_alpha;
   // fused fit + folds (cvmx_fit_folds): raw float64 Gram of every fold of a true partition, [P][ntiles][GACC][GTHREADS],
   // valid while csr_version == fold_gram_version; cvmx_training_batch then only runs statistics + epilogue
   TableCache tc_gram, tc_finish;
@@ -1770,18 +1773,7 @@ int32_t pls_cv_impl(cvmx_t* h, int64_t f0, int64_t f1, int64_t A, void* opress, 
     }
     CU(h, cudaGetLastError());
     // PRESS: chunks of at most PRESS_ROWS validation rows, never spanning two folds; then chunk_off [Pn + 1]
-    tab.clear();
-    std::vector<int64_t> coff((size_t)Pn + 1, 0);
-    for (int64_t f = c0; f < c1; ++f) {
-      for (int64_t p = off[f]; p < off[f + 1]; p += PRESS_ROWS) {
-        tab.push_back(p);
-        tab.push_back(std::min<int64_t>(PRESS_ROWS, off[f + 1] - p));
-        tab.push_back(f - c0);
-      }
-      coff[f - c0 + 1] = (int64_t)tab.size() / 3;
-    }
-    const int64_t nch = (int64_t)tab.size() / 3;
-    tab.insert(tab.end(), coff.begin(), coff.end());
+    const int64_t nch = press_chunk_table(off, c0, c1, tab);
     CU(h, h->pls_tab.reserve(tab.size() * sizeof(int64_t)));
     CU(h, cudaMemcpyAsync(h->pls_tab.p, tab.data(), tab.size() * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
     CU(h, h->pls_part.reserve((size_t)std::max<int64_t>(nch, 1) * (A * M + 1) * sizeof(double)));
@@ -1823,6 +1815,136 @@ int32_t pls_cv_impl(cvmx_t* h, int64_t f0, int64_t f1, int64_t A, void* opress, 
       CU(h, cudaMemcpyAsync((T*)osumw + d, dsumw, (size_t)Pn * sz, kind, h->stream));
       CU(h, cudaMemcpyAsync(ostatus + d, dstatus, (size_t)Pn * sizeof(int32_t), kind, h->stream));
       if (oB) CU(h, cudaMemcpyAsync((char*)oB + (size_t)d * A * K * M * sz, dB, (size_t)Pn * A * K * M * sz, kind, h->stream));
+    }
+    // the next window reuses the scratch and the chunk table's host vector
+    CU(h, cudaStreamSynchronize(h->stream));
+  }
+  return CVMX_OK;
+}
+
+// Cross-validated ridge over folds [f0, f1) (include/cvmx.h: cvmx_ridge_cv).  `plan` is ridge_plan's for this call and
+// is feasible: every scratch size and launch geometry below comes from it.  Per window run_folds leaves the folds' XTX /
+// XTY, statistics and fold scalars in library scratch; per pass of penalties the factorisation, the substitutions and
+// PRESS run over every (fold, penalty) pair.  A pass covers all penalties of its window or a one-fold window, so the
+// outputs of a pass are one contiguous range of the caller's arrays.
+template <typename T>
+int32_t ridge_cv_impl(cvmx_t* h, int64_t f0, int64_t f1, const double* alphas, int64_t L, void* opress, void* osumw, void* oB,
+                      int32_t* oinfo, int32_t* ostatus, int32_t mem, const int64_t* plan) {
+  const size_t sz = sizeof(T);
+  const int64_t K = h->K, M = h->M;
+  const uint32_t want = CVMX_WANT_XTX | CVMX_WANT_XTY;
+  const bool host = mem == CVMX_HOST;
+  const cudaMemcpyKind kind = host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  const int64_t W = plan[CVMX_RIDGE_FOLDS_PER_WINDOW], Lp = plan[CVMX_RIDGE_PENALTIES_PER_PASS];
+  const int64_t G = plan[CVMX_RIDGE_CHUNKS_PER_LAUNCH];
+  const int64_t* grid = plan + CVMX_RIDGE_GRID;
+  const int64_t* smem = plan + CVMX_RIDGE_SMEM;
+  if (f1 <= f0) return CVMX_OK;
+  CU(h, cudaFuncSetAttribute(k_ridge_potrf_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem[CVMX_RK_POTRF]));
+  CU(h, cudaFuncSetAttribute(k_ridge_trsm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem[CVMX_RK_TRSM]));
+  CU(h, cudaFuncSetAttribute(k_ridge_syrk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem[CVMX_RK_SYRK]));
+  CU(h, cudaFuncSetAttribute(k_ridge_bsolve_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem[CVMX_RK_BSOLVE_DIAG]));
+  CU(h, cudaFuncSetAttribute(k_ridge_bsolve_update, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem[CVMX_RK_BSOLVE_UPDATE]));
+  CU(h, cudaFuncSetAttribute(k_ridge_press<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem[CVMX_RK_PRESS]));
+  CU(h, h->ridge_ws.reserve((size_t)plan[CVMX_RIDGE_SCRATCH_BYTES]));
+  CU(h, h->ridge_part.reserve((size_t)plan[CVMX_RIDGE_PART_BYTES]));
+  CU(h, h->ridge_alpha.reserve((size_t)L * sizeof(double)));
+  CU(h, h->out_xx.reserve((size_t)W * K * K * sz));
+  CU(h, h->out_xy.reserve((size_t)W * K * M * sz));
+  // the penalties live on the device before any kernel runs; kernels never see a host address
+  CU(h, cudaMemcpyAsync(h->ridge_alpha.p, alphas, (size_t)L * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  char* ws = h->ridge_ws.as<char>();
+  RidgeState st;
+  st.K = K; st.M = M;
+  st.A = reinterpret_cast<double*>(ws);
+  st.state = reinterpret_cast<int32_t*>(ws + plan[CVMX_RIDGE_END_A]);
+  double* acc = reinterpret_cast<double*>(ws + plan[CVMX_RIDGE_END_STATE]);
+  double* acc_w = reinterpret_cast<double*>(ws + plan[CVMX_RIDGE_END_ACC]);
+  const int64_t* off = h->h_off.data();
+  std::vector<int64_t> tab;
+  for (int64_t c0 = f0; c0 < f1; c0 += W) {
+    const int64_t c1 = std::min(f1, c0 + W), Pn = c1 - c0, d = c0 - f0;
+    int32_t rc = run_folds<T>(h, h->d_off.as<int64_t>(), h->d_idx.as<int64_t>(), off, c0, c1, want, h->out_xx.as<T>(),
+                              h->out_xy.as<T>(), W >= f1 - f0);
+    if (rc) return rc;
+    const int64_t nch = press_chunk_table(off, c0, c1, tab);
+    if (nch > RIDGE_MAX_GRID_X) return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: too many validation rows in one window");
+    CU(h, h->ridge_tab.reserve(std::max<size_t>(tab.size(), 1) * sizeof(int64_t)));
+    CU(h, cudaMemcpyAsync(h->ridge_tab.p, tab.data(), tab.size() * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
+    const int64_t* dtab = h->ridge_tab.as<int64_t>();
+    T* dsumw = host ? reinterpret_cast<T*>(ws + plan[CVMX_RIDGE_END_B]) : (T*)osumw + d;
+    int32_t* dstatus = host ? reinterpret_cast<int32_t*>(ws + plan[CVMX_RIDGE_END_SUM_W]) : ostatus + d;
+    k_pack_scalars<T><<<(unsigned)((Pn + 255) / 256), 256, 0, h->stream>>>(h->fscal.as<FoldScalars>(), Pn, nullptr, dstatus);
+    h->launches++;
+    for (int64_t l0 = 0; l0 < L; l0 += Lp) {
+      const int64_t Lc = std::min(L, l0 + Lp) - l0, pairs = Pn * Lc;
+      if (Pn > 1 && Lc != L) return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: inconsistent launch plan");
+      st.Lp = Lc;
+      const int64_t width = Lc * M;
+      // outputs of the pass: folds [c0, c1) x penalties [l0, l0 + Lc), one contiguous range of the caller's arrays
+      const size_t o_pm = (size_t)(d * L + l0) * M, o_in = (size_t)(d * L + l0), o_b = (size_t)(d * L + l0) * K * M;
+      T* dpress = host ? reinterpret_cast<T*>(ws + plan[CVMX_RIDGE_END_ACC_W]) : (T*)opress + o_pm;
+      int32_t* dinfo = host ? reinterpret_cast<int32_t*>(ws + plan[CVMX_RIDGE_END_PRESS]) : oinfo + o_in;
+      T* dB = !oB ? nullptr : host ? reinterpret_cast<T*>(ws + plan[CVMX_RIDGE_END_INFO]) : (T*)oB + o_b;
+      CU(h, cudaMemsetAsync(acc, 0, (size_t)(plan[CVMX_RIDGE_END_ACC_W] - plan[CVMX_RIDGE_END_STATE]), h->stream));
+      const dim3 gl((unsigned)pairs, (unsigned)grid[2 * CVMX_RK_LOAD + 1]);
+      k_ridge_load<T><<<gl, RIDGE_THREADS, 0, h->stream>>>(h->out_xx.as<T>(), h->out_xy.as<T>(), h->fscal.as<FoldScalars>(), h->flags,
+                                                           h->ridge_alpha.as<double>() + l0, st);
+      h->launches++;
+      for (int64_t j = 0; j < K; j += RIDGE_NB) {
+        const int nbj = (int)std::min<int64_t>(RIDGE_NB, K - j);
+        k_ridge_potrf_diag<<<(unsigned)pairs, RIDGE_THREADS, smem[CVMX_RK_POTRF], h->stream>>>(st, j, nbj);
+        const dim3 gt((unsigned)pairs, (unsigned)ridge_cdiv(K + M - j - nbj, RIDGE_TR_ROWS));
+        k_ridge_trsm<<<gt, RIDGE_TR_ROWS, smem[CVMX_RK_TRSM], h->stream>>>(st, j, nbj);
+        h->launches += 2;
+        if (j + nbj < K) {
+          const SyrkTiles t = ridge_syrk_tiles(K, M, j + nbj);
+          k_ridge_syrk<<<(unsigned)(pairs * t.total), RIDGE_THREADS, smem[CVMX_RK_SYRK], h->stream>>>(st, j, nbj, t);
+          h->launches++;
+        }
+      }
+      for (int64_t j = (K - 1) / RIDGE_NB * RIDGE_NB; j >= 0; j -= RIDGE_NB) {
+        const int nbj = (int)std::min<int64_t>(RIDGE_NB, K - j);
+        k_ridge_bsolve_diag<<<(unsigned)pairs, RIDGE_BS_THREADS, smem[CVMX_RK_BSOLVE_DIAG], h->stream>>>(st, j, nbj);
+        h->launches++;
+        if (j > 0) {
+          const dim3 gu((unsigned)pairs, (unsigned)(j / RIDGE_NB));
+          k_ridge_bsolve_update<<<gu, RIDGE_THREADS, smem[CVMX_RK_BSOLVE_UPDATE], h->stream>>>(st, j, nbj);
+          h->launches++;
+        }
+      }
+      // PRESS over the window's chunks, at most G chunks per launch, each launch's sums added in chunk order
+      for (int64_t g0 = 0; g0 < nch; g0 += G) {
+        const int64_t g1 = std::min(nch, g0 + G);
+        RidgePressParams<T> pp;
+        pp.Z = h->Z.as<T>(); pp.w = h->weighted ? h->w.as<T>() : nullptr; pp.ld = h->ld;
+        pp.idx = h->d_idx.as<int64_t>(); pp.chunks = dtab + 3 * g0; pp.stats = h->stats.as<T>();
+        pp.flags = h->flags; pp.s = st;
+        pp.part = h->ridge_part.as<double>(); pp.part_w = pp.part + (g1 - g0) * width;
+        const dim3 gp((unsigned)(g1 - g0), (unsigned)ridge_cdiv(width, RIDGE_PC));
+        k_ridge_press<T><<<gp, RIDGE_THREADS, smem[CVMX_RK_PRESS], h->stream>>>(pp);
+        const int64_t fa = tab[3 * g0 + 2], fb = tab[3 * (g1 - 1) + 2] + 1;
+        k_ridge_press_accum<<<(unsigned)(fb - fa), RIDGE_THREADS, 0, h->stream>>>(pp.part, pp.part_w, dtab + 3 * nch, g0, g1, fa,
+                                                                                  width, acc, acc_w);
+        h->launches += 2;
+      }
+      k_ridge_finish<T><<<(unsigned)Pn, RIDGE_THREADS, 0, h->stream>>>(st, acc, acc_w, dpress, dinfo, dsumw);
+      h->launches++;
+      if (dB) {
+        const dim3 gc((unsigned)pairs, (unsigned)grid[2 * CVMX_RK_COEFS + 1]);
+        k_ridge_coefs<T><<<gc, RIDGE_THREADS, 0, h->stream>>>(st, dB);
+        h->launches++;
+      }
+      CU(h, cudaGetLastError());
+      if (host) {
+        CU(h, cudaMemcpyAsync((T*)opress + o_pm, dpress, (size_t)pairs * M * sz, kind, h->stream));
+        CU(h, cudaMemcpyAsync(oinfo + o_in, dinfo, (size_t)pairs * sizeof(int32_t), kind, h->stream));
+        if (oB) CU(h, cudaMemcpyAsync((T*)oB + o_b, dB, (size_t)pairs * K * M * sz, kind, h->stream));
+      }
+    }
+    if (host) {
+      CU(h, cudaMemcpyAsync((T*)osumw + d, dsumw, (size_t)Pn * sz, kind, h->stream));
+      CU(h, cudaMemcpyAsync(ostatus + d, dstatus, (size_t)Pn * sizeof(int32_t), kind, h->stream));
     }
     // the next window reuses the scratch and the chunk table's host vector
     CU(h, cudaStreamSynchronize(h->stream));
@@ -1948,7 +2070,7 @@ int32_t cvmx_destroy(cvmx_t* h) {
   for (DevBuf* b : {&h->stat_flags, &h->peer_sum, &h->w_glob, &h->g_off, &h->g_idx, &h->scan_look, &h->loo_ops, &h->Z, &h->w, &h->Ttot, &h->sum_z, &h->sumsq_z, &h->fit_scal, &h->d_off, &h->d_idx, &h->a_off, &h->a_idx,
                     &h->units, &h->tiles, &h->fold_units, &h->split_folds, &h->partials, &h->stats, &h->rawsums, &h->fscal, &h->pwcols,
                     &h->errflag, &h->out_xx, &h->out_xy, &h->out_small, &h->scan_seg, &h->scan_ok, &h->scan_list, &h->scan_cnt, &h->ystage, &h->fold_gram, &h->fold_raw, &h->chunk_ranges,
-                    &h->pls_ws, &h->pls_tab, &h->pls_part, &h->pls_out})
+                    &h->pls_ws, &h->pls_tab, &h->pls_part, &h->pls_out, &h->ridge_ws, &h->ridge_tab, &h->ridge_part, &h->ridge_alpha})
     b->release();
   h->tc_gram.release(); h->tc_finish.release();
   delete h->stager; h->stager = nullptr;
@@ -2401,6 +2523,38 @@ int32_t cvmx_pls_cv(cvmx_t* h, int64_t f0, int64_t f1, int64_t n_components, voi
   return h->dtype == CVMX_F64
              ? pls_cv_impl<double>(h, f0, f1, n_components, out_press, out_sum_w_val, out_B, out_n_fitted, out_status, mem)
              : pls_cv_impl<float>(h, f0, f1, n_components, out_press, out_sum_w_val, out_B, out_n_fitted, out_status, mem);
+}
+
+int32_t cvmx_ridge_plan(int64_t K, int64_t M, int64_t L, int64_t P, int32_t dtype, int32_t mem, int32_t want_B, int64_t* plan) {
+  if (!plan) return fail(nullptr, CVMX_ERR_INVALID, "cvmx_ridge_plan: plan is NULL");
+  const int32_t rc = ridge_plan(K, M, L, P, dtype, mem, want_B, plan);
+  return rc ? fail(nullptr, rc, "cvmx_ridge_plan: the shape cannot run within the device limits") : CVMX_OK;
+}
+
+int32_t cvmx_ridge_cv(cvmx_t* h, int64_t f0, int64_t f1, const double* alphas, int64_t L, void* out_press, void* out_sum_w_val,
+                      void* out_B, int32_t* out_info, int32_t* out_status, int32_t mem) {
+  if (!h || !h->fitted) return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: fit first");
+  if (h->slab) return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: not available for a row-slab handle");
+  if (f0 < 0 || f1 > h->P || f0 > f1) return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: fold range outside the CSR");
+  if (h->M == 0) return fail(h, CVMX_ERR_NO_Y, "Response variables `Y` are not provided.");
+  if (h->M > RIDGE_MAX_M)
+    return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: at most " + std::to_string(RIDGE_MAX_M) + " response columns are supported");
+  if (!alphas || L < 1 || L > RIDGE_MAX_L)
+    return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: alphas must hold between 1 and " + std::to_string(RIDGE_MAX_L) + " penalties");
+  for (int64_t l = 0; l < L; ++l)
+    if (!(alphas[l] >= 0.0 && alphas[l] <= 1.7976931348623157e308))
+      return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: every penalty must be finite and >= 0");
+  if (mem != CVMX_HOST && mem != CVMX_DEVICE) return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: mem must be CVMX_HOST or CVMX_DEVICE");
+  if (f1 > f0 && (!out_press || !out_sum_w_val || !out_info || !out_status))
+    return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: an output pointer is NULL");
+  int64_t plan[CVMX_RIDGE_PLAN_LEN];
+  if (ridge_plan(h->K, h->M, L, f1 - f0, h->dtype, mem, out_B != nullptr, plan) != CVMX_OK || plan[CVMX_RIDGE_FEASIBLE] != 1)
+    return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: K = " + std::to_string(h->K) + ", M = " + std::to_string(h->M) +
+                                         " cannot run within the device limits");
+  ON_DEVICE(h);
+  return h->dtype == CVMX_F64
+             ? ridge_cv_impl<double>(h, f0, f1, alphas, L, out_press, out_sum_w_val, out_B, out_info, out_status, mem, plan)
+             : ridge_cv_impl<float>(h, f0, f1, alphas, L, out_press, out_sum_w_val, out_B, out_info, out_status, mem, plan);
 }
 
 int32_t cvmx_profile_enable(cvmx_t* h, int32_t on) {

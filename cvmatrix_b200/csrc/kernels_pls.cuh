@@ -10,6 +10,7 @@
 // k_pls_press_reduce (chunks of a fold summed in chunk order), and k_pls_coefs when B is wanted.
 // Every reduction has a fixed order that depends on the problem only, never on the grid: two calls give the same bits.
 #pragma once
+#include <vector>
 #include "common.cuh"
 
 namespace cvmx {
@@ -403,6 +404,33 @@ __global__ void __launch_bounds__(PLS_THREADS) k_pls_press(PressParams<T> p) {
   }
 }
 
+// PRESS chunks of folds [c0, c1) of the CSR (host offsets `off`): at most PRESS_ROWS validation rows each, never
+// spanning two folds.  tab = [nch][3] {first CSR position, rows, fold - c0}, then chunk_off [c1 - c0 + 1] (first chunk of
+// every fold); returns nch.
+inline int64_t press_chunk_table(const int64_t* off, int64_t c0, int64_t c1, std::vector<int64_t>& tab) {
+  tab.clear();
+  std::vector<int64_t> coff((size_t)(c1 - c0) + 1, 0);
+  for (int64_t f = c0; f < c1; ++f) {
+    for (int64_t p = off[f]; p < off[f + 1]; p += PRESS_ROWS) {
+      tab.push_back(p);
+      tab.push_back(off[f + 1] - p < PRESS_ROWS ? off[f + 1] - p : PRESS_ROWS);
+      tab.push_back(f - c0);
+    }
+    coff[f - c0 + 1] = (int64_t)tab.size() / 3;
+  }
+  const int64_t nch = (int64_t)tab.size() / 3;
+  tab.insert(tab.end(), coff.begin(), coff.end());
+  return nch;
+}
+
+// t + part[c0][e] + part[c0 + 1][e] + ... + part[c1 - 1][e] (row pitch `width`), added in chunk order: the PRESS of a
+// fold does not depend on how its chunks were spread over CTAs or launches.
+__device__ __forceinline__ double press_chunk_sum(const double* __restrict__ part, int64_t width, int64_t c0, int64_t c1, int64_t e,
+                                                  double t) {
+  for (int64_t c = c0; c < c1; ++c) t += part[c * width + e];
+  return t;
+}
+
 // press[f][a][m] = sum of the fold's chunk partials in chunk order (NaN for refused folds), sum_w_val[f] likewise.
 // chunk_off: [Pn + 1] first chunk of every fold.  One block per fold.
 template <typename T>
@@ -413,16 +441,8 @@ __global__ void __launch_bounds__(PLS_THREADS) k_pls_press_reduce(const double* 
   const int64_t c0 = chunk_off[f], c1 = chunk_off[f + 1];
   const bool bad = s.state[f] == PLS_BAD;
   const double nan = __longlong_as_double(0x7ff8000000000000LL);
-  for (int64_t e = threadIdx.x; e < AM; e += PLS_THREADS) {
-    double t = 0.0;
-    for (int64_t c = c0; c < c1; ++c) t += part[c * AM + e];
-    press[f * AM + e] = (T)(bad ? nan : t);
-  }
-  if (threadIdx.x == 0) {
-    double t = 0.0;
-    for (int64_t c = c0; c < c1; ++c) t += part_w[c];
-    sum_w[f] = (T)t;
-  }
+  for (int64_t e = threadIdx.x; e < AM; e += PLS_THREADS) press[f * AM + e] = (T)(bad ? nan : press_chunk_sum(part, AM, c0, c1, e, 0.0));
+  if (threadIdx.x == 0) sum_w[f] = (T)press_chunk_sum(part_w, 1, c0, c1, 0, 0.0);
 }
 
 }  // namespace cvmx

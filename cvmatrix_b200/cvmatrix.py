@@ -624,6 +624,94 @@ class CVMatrix:
                           UserWarning, stacklevel=2)
         return dict(press=press, sum_w_val=sum_w, n_fitted=n_fitted, status=status, B=B)
 
+    def ridge_cross_validate(self, alphas, fold_begin: int = 0, fold_end: Optional[int] = None, return_coefs: bool = False,
+                             out: str = "numpy", check: bool = True):
+        """
+        Cross-validated ridge regression over folds ``[fold_begin, fold_end)`` of the CSR (see ``set_folds``) for every
+        penalty in ``alphas``, on the GPU.
+
+        Per fold and penalty ``lam``: ``B = (XTX + lam I)^-1 XTY`` by a blocked Cholesky factorisation in float64, from the
+        fold's ``XTX`` / ``XTY`` and training statistics exactly as ``training_batch`` forms them.  ``lam`` is added to the
+        diagonal of the matrix as formed: with ``scale_X`` it penalises the coefficients of the standardised X columns,
+        and with ``center_X`` / ``center_Y`` the intercept is not penalised (scikit-learn's ``Ridge(fit_intercept=True)``).
+        The fold's validation rows are predicted as ``((x - X_mean) / X_std) @ B * Y_std + Y_mean`` (each statistic
+        applied iff its flag is set) and scored.  ``alphas`` is a 1-D host sequence of 1 to 1024 finite penalties >= 0
+        (repeats allowed).
+
+        Returns a dict with ``press`` (P, L, M): the weighted sum of squared prediction errors over the validation rows,
+        ``sum_w_val`` (P,): the sum of their weights (their count when unweighted), ``info`` (P, L) int32: 0, or the
+        1-based column of the first pivot that was not positive (as LAPACK ``dpotrf`` reports it), ``status`` (P,) int32
+        (``CVMX_FOLD_*`` bits) and ``B`` (P, L, K, M) with ``return_coefs``, else None.  A pair with ``info != 0`` gets NaN
+        ``press`` / ``B``; a ``UserWarning`` counts such pairs (``lam = 0`` on a rank-deficient fold is a legitimate grid
+        point, not an error).  ``out="torch"`` returns CUDA tensors, ``out="numpy"`` host arrays.  With ``check`` the
+        degenerate fold errors of ``training_XTX_XTY`` are raised; without it such folds get NaN ``press`` / ``B`` for
+        every penalty and ``info`` 0.
+
+        Example - root mean squared error of cross-validation per penalty and response::
+
+            cvm.fit(X, Y); cvm.set_folds(Partitioner(folds))
+            r = cvm.ridge_cross_validate(np.logspace(-3, 3, 20))
+            rmsecv = np.sqrt(r["press"].sum(0) / r["sum_w_val"].sum())    # (L, M)
+        """
+        self._require_fit()
+        if fold_end is None:
+            fold_end = self._n_folds
+        if not self._has_Y:
+            raise ValueError(_ERR_NO_Y)
+        if hasattr(alphas, "detach"):   # a torch tensor: the penalties are read on the host
+            alphas = alphas.detach().cpu().numpy()
+        try:
+            lam = np.ascontiguousarray(np.asarray(alphas, dtype=np.float64))
+        except (TypeError, ValueError):
+            raise ValueError("alphas must be a 1-D sequence of finite penalties >= 0") from None
+        if lam.ndim != 1 or not 1 <= lam.size <= 1024:
+            raise ValueError(f"alphas must be a 1-D sequence of 1 to 1024 penalties; got shape {lam.shape}")
+        if not (np.isfinite(lam).all() and (lam >= 0).all()):
+            raise ValueError("every penalty in alphas must be finite and >= 0")
+        L, K, M, dt = lam.size, self.K, self.M, self.dtype
+        if M > 128:
+            raise ValueError(f"at most 128 response columns are supported; Y has {M}")
+        P = max(int(fold_end) - int(fold_begin), 0)
+        if out == "torch":
+            import torch
+
+            tdt = torch.float64 if np.dtype(dt) == np.float64 else torch.float32
+            dev = torch.device("cuda", self.device)
+            press = torch.empty((P, L, M), dtype=tdt, device=dev)
+            sum_w = torch.empty((P,), dtype=tdt, device=dev)
+            info = torch.empty((P, L), dtype=torch.int32, device=dev)
+            status = torch.empty((P,), dtype=torch.int32, device=dev)
+            B = torch.empty((P, L, K, M), dtype=tdt, device=dev) if return_coefs else None
+            p, mem = _tptr, _lib.DEVICE
+        elif out == "numpy":
+            press = np.empty((P, L, M), dt)
+            sum_w = np.empty((P,), dt)
+            info = np.zeros((P, L), np.int32)
+            status = np.zeros((P,), np.int32)
+            B = np.empty((P, L, K, M), dt) if return_coefs else None
+            p, mem = _ptr, _lib.HOST
+        else:
+            raise ValueError("out must be 'numpy' or 'torch'")
+        with self._torch_stream() if out == "torch" else contextlib.nullcontext():
+            rc = self._lib.cvmx_ridge_cv(self._h, int(fold_begin), int(fold_end), _ptr(lam), L, p(press), p(sum_w), p(B),
+                                         p(info), p(status), mem)
+            _lib.check(rc, self._h)
+        if check:
+            st = status.cpu().numpy() if out == "torch" else status
+            cX, cY, sX, sY = self.center_X, self.center_Y, self.scale_X, self.scale_Y
+            need = (cX or cY, sX, cX or cY, sY)    # the statistics training_XTX_XTY computes
+            for s in np.unique(st):
+                if s:
+                    self._raise_for_status(int(s), need)
+        inf = info.cpu().numpy() if out == "torch" else info
+        failed = np.argwhere(inf != 0)
+        if failed.size:
+            f, l = (int(x) for x in failed[0])
+            warnings.warn(f"{len(failed)} (fold, penalty) pair(s) could not be factored: XTX + alpha I is not positive "
+                          f"definite (first: fold {int(fold_begin) + f}, alpha {lam[l]!r} at index {l}, pivot {int(inf[f, l])}); "
+                          "their press and B are NaN", UserWarning, stacklevel=2)
+        return dict(press=press, sum_w_val=sum_w, info=info, status=status, B=B)
+
     def validation_rows(self, fold: int, stats: Optional[Stats] = None, out: str = "numpy"):
         """
         ``(X[val], Y[val])`` of CSR fold number ``fold`` (see ``set_folds``) for the caller's next step - predicting the

@@ -291,6 +291,57 @@ int32_t cvmx_validation_rows(cvmx_t* h, int64_t fold, const void* stats, uint32_
 int32_t cvmx_pls_cv(cvmx_t* h, int64_t fold_begin, int64_t fold_end, int64_t n_components, void* out_press,
                     void* out_sum_w_val, void* out_B, int32_t* out_n_fitted, int32_t* out_status, int32_t mem);
 
+/*
+ * Cross-validated ridge regression over folds [fold_begin, fold_end) of the CSR for L penalties - the other linear model
+ * fitted from the training matrices (the caller's per-fold np.linalg.solve(XTX + lambda I, XTY) after
+ * training_XTX_XTY, cvmatrix/partitioner.py:27-31).  Per fold f and penalty lambda_l = alphas[l] (a HOST array of L
+ * finite values >= 0, 1 <= L <= 1024; copied to the device once per call), from XTX / XTY and the statistics exactly
+ * as cvmx_training_batch(XTX | XTY) forms them: B = (XTX + lambda_l I)^-1 XTY by a blocked Cholesky factorisation in
+ * float64 (lambda is added to the diagonal of the matrix as formed, so with scale_X it penalises the standardised
+ * coefficients), then the validation rows x_i of the fold predict y^_i = ((x_i - mu_X) / sigma_X) B * sigma_Y + mu_Y
+ * (each statistic applied iff its flag is set).  With P' = fold_end - fold_begin, in the handle's dtype unless noted:
+ *   out_press      [P', L, M]     sum over the validation rows (as stored: repeats count) of w_i (y_im - y^_im)^2
+ *   out_sum_w_val  [P']           sum of the validation weights (row count when unweighted)
+ *   out_B          [P', L, K, M]  coefficients (may be NULL)
+ *   out_info       [P', L] int32  0, or the 1-based column of the first pivot that was not > 0 (NaN included), as
+ *                                 LAPACK dpotrf reports it; such a pair gets NaN press and B
+ *   out_status     [P'] int32     CVMX_FOLD_* bits
+ * Folds whose status bits make training_XTX_XTY raise (cvmatrix/cvmatrix.py:625-629, 1074-1078) get NaN press and B for
+ * every penalty and info 0.  Folds are processed in windows and the penalties of a window in passes, as
+ * cvmx_ridge_plan says; a range that fits one window reuses the fold Grams kept by cvmx_fit_folds.  M = 0 gives
+ * CVMX_ERR_NO_Y; M > 128, a bad penalty list, a row-slab handle or a shape cvmx_ridge_plan calls infeasible give
+ * CVMX_ERR_INVALID before anything is launched.  `mem` applies to all five outputs.  Results do not depend on the launch
+ * geometry, the windows or the passes: identical calls give identical bits.
+ */
+int32_t cvmx_ridge_cv(cvmx_t* h, int64_t fold_begin, int64_t fold_end, const double* alphas, int64_t L, void* out_press,
+                      void* out_sum_w_val, void* out_B, int32_t* out_info, int32_t* out_status, int32_t mem);
+
+/* Host-only (no CUDA call): the launch plan cvmx_ridge_cv uses for K columns of X, M of Y, L penalties and P folds of
+ * the given dtype, output memory (`mem`) and whether B is wanted.  plan[CVMX_RIDGE_PLAN_LEN] receives the folds per
+ * window, the penalties per pass, the device scratch bytes of a pass and the byte offset at which each of its arrays
+ * ends, the PRESS partials of one launch, the largest grid (x, y) of every kernel (CVMX_RIDGE_GRID + 2 * CVMX_RK_*) and
+ * its dynamic shared memory (CVMX_RIDGE_SMEM + CVMX_RK_*).  A pass holds every penalty of its folds, or one fold.
+ * Returns CVMX_OK with plan[CVMX_RIDGE_FEASIBLE] = 1, or CVMX_ERR_INVALID (feasible = 0) for arguments out of range or a
+ * shape that cannot run within the device limits (grid dimensions, 227 KB of shared memory a block, 32 GiB of scratch
+ * for one fold and one penalty). */
+int32_t cvmx_ridge_plan(int64_t K, int64_t M, int64_t L, int64_t P, int32_t dtype, int32_t mem, int32_t want_B, int64_t* plan);
+
+enum {
+  CVMX_RK_LOAD = 0, CVMX_RK_POTRF, CVMX_RK_TRSM, CVMX_RK_SYRK, CVMX_RK_BSOLVE_DIAG, CVMX_RK_BSOLVE_UPDATE,
+  CVMX_RK_PRESS, CVMX_RK_PRESS_ACCUM, CVMX_RK_FINISH, CVMX_RK_COEFS, CVMX_RK_COUNT
+};
+enum {
+  CVMX_RIDGE_FEASIBLE = 0, CVMX_RIDGE_FOLDS_PER_WINDOW, CVMX_RIDGE_PENALTIES_PER_PASS, CVMX_RIDGE_SCRATCH_BYTES,
+  CVMX_RIDGE_END_A, CVMX_RIDGE_END_STATE, CVMX_RIDGE_END_ACC, CVMX_RIDGE_END_ACC_W, CVMX_RIDGE_END_PRESS,
+  CVMX_RIDGE_END_INFO, CVMX_RIDGE_END_B, CVMX_RIDGE_END_SUM_W, CVMX_RIDGE_END_STATUS,
+  CVMX_RIDGE_WINDOW_BYTES,       /* XTX / XTY of one window (model dtype) */
+  CVMX_RIDGE_PART_BYTES,         /* PRESS partials of one launch */
+  CVMX_RIDGE_CHUNKS_PER_LAUNCH,  /* PRESS chunks of one launch */
+  CVMX_RIDGE_GRID = 16,
+  CVMX_RIDGE_SMEM = CVMX_RIDGE_GRID + 2 * CVMX_RK_COUNT,
+  CVMX_RIDGE_PLAN_LEN = CVMX_RIDGE_SMEM + CVMX_RK_COUNT
+};
+
 /* Per-kernel device timing for bench.py's roofline line: while enabled, CUDA events are recorded on the
  * handle's stream around the statistics kernels (ms[0]), the Gram kernel (ms[1]) and the split-reduce
  * kernel (ms[2]); cvmx_profile_read synchronises, returns the accumulated milliseconds and span counts
