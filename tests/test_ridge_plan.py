@@ -76,6 +76,24 @@ def test_both_splits_occur():
     assert rc == _lib.OK and p[_lib.RIDGE_FOLDS_PER_WINDOW] == 1 and p[_lib.RIDGE_PENALTIES_PER_PASS] == 1024
 
 
+def test_splits_of_the_edge_shapes():
+    from cvmatrix_b200 import _lib
+
+    # the shapes tests/test_gpu_cv_edges.py uses, for host and device outputs, with and without B
+    for mem, want_B in itertools.product((0, 1), (0, 1)):
+        # PRESS over several launches: 131,072 columns leave 255 chunks per launch; two folds of 313 chunks need three
+        rc, p = _plan(4, 128, 1024, 2, mem=mem, want_B=want_B)
+        assert rc == _lib.OK and p[_lib.RIDGE_FOLDS_PER_WINDOW] == 2 and p[_lib.RIDGE_PENALTIES_PER_PASS] == 1024
+        assert p[_lib.RIDGE_CHUNKS_PER_LAUNCH] == 255
+        # leave-one-out over 595 folds: three to five windows of all 16 penalties
+        rc, p = _plan(200, 8, 16, 595, mem=mem, want_B=want_B)
+        W = p[_lib.RIDGE_FOLDS_PER_WINDOW]
+        assert rc == _lib.OK and p[_lib.RIDGE_PENALTIES_PER_PASS] == 16 and 3 <= -(-595 // W) <= 5
+        # one fold per window, its penalties in passes
+        rc, p = _plan(400, 2, 1024, 3, mem=mem, want_B=want_B)
+        assert rc == _lib.OK and p[_lib.RIDGE_FOLDS_PER_WINDOW] == 1 and 1 < p[_lib.RIDGE_PENALTIES_PER_PASS] < 1024
+
+
 def test_infeasible_and_invalid_shapes():
     from cvmatrix_b200 import _lib
 
