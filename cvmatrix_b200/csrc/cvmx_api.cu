@@ -216,7 +216,7 @@ void plan_tiles(const cvmx_t* h, uint32_t want, std::vector<int2>& tiles) {
   tiles.clear();
   const int64_t TI = (h->K + GB - 1) / GB, TJ = (h->K + h->M + GB - 1) / GB;
   // Diagonal tiles first (and the tiles (0, bj >= TI) of Y-only column blocks): with fused fold statistics every tile of a
-  // fold waits for their column chains before its epilogue - started first, and the diagonal ones issuing 3/4 of the DMMAs
+  // fold waits for their column chains before its epilogue - started first, and the diagonal ones issuing 9/16 of the DMMAs
   // of a full tile, they are done before the others need them.
   for (int pass = 0; pass < 2; ++pass)
     for (int64_t bi = 0; bi < TI; ++bi)
@@ -233,8 +233,9 @@ void plan_tiles(const cvmx_t* h, uint32_t want, std::vector<int2>& tiles) {
 // The hardware places CTAs greedily (next CTA to the first SM that frees up), so equal-sized units end in a ragged last
 // wave: 1150 equal items on 148 SMs leave a quarter of the GPU idle for a whole item.  Unit sizes therefore TAPER - a few
 // long units, then halves, quarters, ... - and are launched longest first, which is the classic LPT packing; the sizes
-// are chosen by simulating that placement with the measured relative tile costs (a diagonal tile issues 3/4 of the
-// DMMAs of a full one; ~1.5 pipeline stages of fixed cost per CTA).  Returns per fold the unit sizes in split order.
+// are chosen by simulating that placement with the measured relative tile costs (a diagonal tile issues 9/16 of the
+// DMMAs of a full one and takes 0.79 of its time, measured by tools/tile_cost.py over the same row-split units; ~1.5
+// pipeline stages of fixed cost per CTA).  Returns per fold the unit sizes in split order.
 double simulate_makespan(std::vector<int64_t> unit_rows, const std::vector<double>& tile_cost, int64_t sms) {
   std::sort(unit_rows.begin(), unit_rows.end(), std::greater<int64_t>());
   std::vector<double> heap((size_t)sms, 0.0);   // min-heap of SM finish times
@@ -281,7 +282,7 @@ std::vector<std::vector<int64_t>> plan_tapered(const std::vector<int64_t>& fold_
   for (const Memo& m : memo)
     if (m.rows == fold_rows && m.ntiles == tiles.size() && m.sms == sms) return m.sizes;
   std::vector<double> tile_cost;
-  for (const int2& t : tiles) tile_cost.push_back(t.x == t.y ? 0.78 : 1.0);
+  for (const int2& t : tiles) tile_cost.push_back(t.x == t.y ? 0.79 : 1.0);
   double best = 1e300;
   std::vector<std::vector<int64_t>> best_sizes;
   for (int64_t R = r_lo; R <= r_hi; R += 8 * GBK)

@@ -271,10 +271,148 @@ __device__ __forceinline__ void gram_epilogue(double (&acc)[8][4][2], T* sC, con
   }
 }
 
+// ---- fragment bands ------------------------------------------------------------------------------------------------
+// A warp tile (64 x 32) is 4 x 2 bands of 16 x 16: band (tp, up) holds the fragments t in {2tp, 2tp + 1} x u in
+// {2up, 2up + 1} (fragment rows interleave inside a band, so a band is the smallest unit a warp can skip).  A band mask
+// selects bands by bit 2 * tp + up.
+constexpr int GBANDS_ALL = 0xFF;
+// Diagonal tiles need only the 36 of their 64 bands that lie on or above the diagonal; a band on the diagonal is
+// computed in full.  They are spread 9 per SM sub-partition (warp % 4), the DMMA issue limit, against 16 in an
+// off-diagonal tile: warp w computes the bands GDIAG_MASK[w] of its own warp tile, except that warp 4 (no band of its
+// own) takes rows 0-47 of the tile of warp GDIAG_OWNER4 = 3 and warp 5 rows 0-15 of the tile of warp GDIAG_OWNER5 = 2.
+// Without the two moves the sub-partitions would carry 3, 7, 11 and 15 bands.
+constexpr int GDIAG_MASK[8] = {0x0B, 0xBF, 0xFC, 0xC0, 0x3F, 0x03, 0x0B, 0xBF};
+constexpr int GDIAG_OWNER4 = 3, GDIAG_OWNER5 = 2;
+constexpr bool gdiag_bands_ok() {
+  int cover[8][8] = {}, smsp[4] = {};
+  for (int w = 0; w < 8; ++w) {
+    const int tile = w == 4 ? GDIAG_OWNER4 : w == 5 ? GDIAG_OWNER5 : w;
+    for (int band = 0; band < 8; ++band)
+      if ((GDIAG_MASK[w] >> band) & 1) {
+        ++cover[(tile >> 2) * 4 + band / 2][(tile & 3) * 2 + band % 2];
+        ++smsp[w % 4];
+      }
+  }
+  for (int r = 0; r < 8; ++r)
+    for (int c = 0; c < 8; ++c)
+      if (cover[r][c] != (r <= c ? 1 : 0)) return false;
+  for (int s = 0; s < 4; ++s)
+    if (smsp[s] != 9) return false;
+  return GDIAG_MASK[6] == GDIAG_MASK[0] && GDIAG_MASK[7] == GDIAG_MASK[1];   // k_gram runs warps 6, 7 on the code of 0, 1
+}
+static_assert(gdiag_bands_ok(), "diagonal-tile bands: each band on or above the diagonal exactly once, 9 per sub-partition");
+
+template <int MASK> __device__ __forceinline__ constexpr bool gram_band(int t, int u) { return (MASK >> ((t >> 1) * 2 + (u >> 1))) & 1; }
+
+// One compute warp's row loop: every pipeline stage of the unit, the fragments of the bands in MASK of the warp tile at
+// tile rows r0 .. r0 + 63 and columns c0 .. c0 + 31.  A band outside MASK costs no DMMA, no fragment load and no rn(w*x).
+template <typename T, int MASK>
+__device__ __forceinline__ void gram_rows(double (&acc)[8][4][2], const T* sA, const T* sB, const T* sW, uint64_t* full,
+                                          uint64_t* empty, int64_t nrows, int r0, int c0) {
+  constexpr int PITCH = GramCfg<T>::PITCH;
+  typedef typename GramCfg<T>::vec2 vec2;
+  const int lane = threadIdx.x & 31, g = lane >> 2, q = lane & 3;
+#pragma unroll 1
+  for (int64_t kt = 0; kt * GBK < nrows; ++kt) {
+    const int slot = (int)(kt % GSTAGES);
+    mbar_wait(full + slot, (unsigned)(kt / GSTAGES) & 1);
+    const T* a_base = sA + (size_t)slot * GBK * PITCH + r0 + 2 * g;
+    const T* b_base = sB + (size_t)slot * GBK * PITCH + c0 + 2 * g;
+    const T* w_base = sW + slot * GBK;
+    const int rows = (int)min((int64_t)GBK, nrows - kt * GBK);
+    if (rows == GBK) {
+#pragma unroll
+      for (int kk = 0; kk < GBK / 4; ++kk) {
+        const int k = kk * 4 + q;
+        const T wv = w_base[k];
+        double a[8], b[4];
+#pragma unroll
+        for (int tp = 0; tp < 4; ++tp) {
+          if (!((MASK >> (2 * tp)) & 3)) continue;
+          const vec2 v = *reinterpret_cast<const vec2*>(a_base + k * PITCH + tp * 16);
+          a[2 * tp] = (double)Rn<T>::mul(v.x, wv);       // rn(w*x) in the model dtype == WX of the reference
+          a[2 * tp + 1] = (double)Rn<T>::mul(v.y, wv);
+        }
+#pragma unroll
+        for (int up = 0; up < 2; ++up) {
+          if (!(MASK & (0x55 << up))) continue;
+          const vec2 v = *reinterpret_cast<const vec2*>(b_base + k * PITCH + up * 16);
+          b[2 * up] = (double)v.x;
+          b[2 * up + 1] = (double)v.y;
+        }
+#pragma unroll
+        for (int t = 0; t < 8; ++t)
+#pragma unroll
+          for (int u = 0; u < 4; ++u)
+            if (gram_band<MASK>(t, u)) dmma884(acc[t][u][0], acc[t][u][1], a[t], b[u]);
+      }
+    } else {
+      // tail stage: rows past the end of the unit were never copied - feed exact zeros instead
+#pragma unroll 1
+      for (int kk = 0; kk * 4 < rows; ++kk) {
+        const int k = kk * 4 + q;
+        const bool ok = k < rows;
+        const T wv = ok ? w_base[k] : T(0);
+        double a[8], b[4];
+#pragma unroll
+        for (int tp = 0; tp < 4; ++tp) {
+          if (!((MASK >> (2 * tp)) & 3)) continue;
+          vec2 v; v.x = T(0); v.y = T(0);
+          if (ok) v = *reinterpret_cast<const vec2*>(a_base + k * PITCH + tp * 16);
+          a[2 * tp] = ok ? (double)Rn<T>::mul(v.x, wv) : 0.0;
+          a[2 * tp + 1] = ok ? (double)Rn<T>::mul(v.y, wv) : 0.0;
+        }
+#pragma unroll
+        for (int up = 0; up < 2; ++up) {
+          if (!(MASK & (0x55 << up))) continue;
+          vec2 v; v.x = T(0); v.y = T(0);
+          if (ok) v = *reinterpret_cast<const vec2*>(b_base + k * PITCH + up * 16);
+          b[2 * up] = (double)v.x;
+          b[2 * up + 1] = (double)v.y;
+        }
+#pragma unroll
+        for (int t = 0; t < 8; ++t)
+#pragma unroll
+          for (int u = 0; u < 4; ++u)
+            if (gram_band<MASK>(t, u)) dmma884(acc[t][u][0], acc[t][u][1], a[t], b[u]);
+      }
+    }
+    __syncwarp();
+    if (lane == 0) mbar_arrive(empty + slot);
+  }
+}
+
+// Bands MASK of the accumulators to / from a lane-interleaved [GACC][32] shared-memory slot (buf = slot + lane).  The
+// sender zeroes what it sent; the receiver computed nothing in those bands and takes the values as they are.
+template <int MASK>
+__device__ __forceinline__ void gram_bands_out(double (&acc)[8][4][2], double* buf) {
+#pragma unroll
+  for (int t = 0; t < 8; ++t)
+#pragma unroll
+    for (int u = 0; u < 4; ++u)
+      if (gram_band<MASK>(t, u)) {
+        buf[((t * 4 + u) * 2 + 0) * 32] = acc[t][u][0];
+        buf[((t * 4 + u) * 2 + 1) * 32] = acc[t][u][1];
+        acc[t][u][0] = acc[t][u][1] = 0.0;
+      }
+}
+template <int MASK>
+__device__ __forceinline__ void gram_bands_in(double (&acc)[8][4][2], const double* buf) {
+#pragma unroll
+  for (int t = 0; t < 8; ++t)
+#pragma unroll
+    for (int u = 0; u < 4; ++u)
+      if (gram_band<MASK>(t, u)) {
+        acc[t][u][0] = buf[((t * 4 + u) * 2 + 0) * 32];
+        acc[t][u][1] = buf[((t * 4 + u) * 2 + 1) * 32];
+      }
+}
+
 // Main kernel, warp-specialised.  Data movement is done by the TMA engine: per pipeline stage, the 32 lanes of a
 // producer warp (warps 8-11 take the stages round-robin) each issue one 1-KB bulk async copy (cp.async.bulk, SASS UBLKCP) of a gathered row segment
 // - 16 rows x {A block, B block} - plus an 8-byte cp.async of the row weight, all completing on the stage's "full"
-// mbarrier.  The eight compute warps wait on that barrier, run 4 x 32 DMMA.8x8x4 on the stage and release it through
+// mbarrier.  The eight compute warps wait on that barrier, run 4 x 32 DMMA.8x8x4 on the stage (a diagonal tile: only the
+// fragment bands of GDIAG_MASK, at most 4 x 36 per sub-partition) and release it through
 // the "empty" mbarrier; there is no block-wide barrier in the main loop and no compute warp ever issues a copy
 // (with the producer role on a compute warp the ~1300 issue cycles per stage sat on the critical path: ncu showed
 // 20 % of all samples in the full-barrier wait).  Row indices are fetched one stage ahead of their use.
@@ -282,7 +420,6 @@ template <typename T, bool FUSE = false>   // FUSE: fused fold statistics (GramP
 __global__ void __launch_bounds__(GLAUNCH, 1) k_gram(const GramParams<T> p) {   // the plain kernel keeps its registers and schedule
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int PITCH = GramCfg<T>::PITCH;
-  typedef typename GramCfg<T>::vec2 vec2;
 
   T* sA = reinterpret_cast<T*>(smem_raw);
   T* sB = sA + (size_t)GSTAGES * GBK * PITCH;
@@ -291,7 +428,7 @@ __global__ void __launch_bounds__(GLAUNCH, 1) k_gram(const GramParams<T> p) {   
   uint64_t* empty = full + GSTAGES;
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int wm = warp >> 2, wn = warp & 3, g = lane >> 2, q = lane & 3;
+  const int wm = warp >> 2, wn = warp & 3;
   const int tile = blockIdx.x % p.ntiles;
   const GramUnit unit = p.units[blockIdx.x / p.ntiles];
   const int2 tl = p.tiles[tile];
@@ -401,83 +538,25 @@ __global__ void __launch_bounds__(GLAUNCH, 1) k_gram(const GramParams<T> p) {   
 #pragma unroll
     for (int u = 0; u < 4; ++u) acc[t][u][0] = acc[t][u][1] = 0.0;
 
-  // Diagonal tiles only need their upper triangle: the warp tiles (rows 64-127) x (cols 0-63) of warps 4 and 5 are
-  // never used.  Those two warps instead help warps 6 and 7 - which sit on the other two sub-partitions - by taking
-  // every other pipeline stage of their tiles (intra-CTA split-K), so each sub-partition carries 1.5 instead of 2
-  // warp-tiles of DMMA work; the two partial accumulators are added through shared memory before the epilogue.
-  const bool half = diag && wm == 1;                 // this warp computes every other stage
-  const bool helper = half && wn < 2;                // ... of the tile of warp (1, wn + 2)
-  const int ewn = helper ? wn + 2 : wn;
-  const int my_parity = helper ? 1 : 0;
-
-#pragma unroll 1
-  for (int64_t kt = 0; kt < nk; ++kt) {
-    const int slot = (int)(kt % GSTAGES);
-    mbar_wait(full + slot, (unsigned)(kt / GSTAGES) & 1);
-    const T* a_base = sA + (size_t)slot * GBK * PITCH + wm * 64 + 2 * g;
-    const T* b_base = (diag ? sA : sB) + (size_t)slot * GBK * PITCH + ewn * 32 + 2 * g;
-    const T* w_base = sW + slot * GBK;
-    const int rows = (int)min((int64_t)GBK, nrows - kt * GBK);
-    if (half && (int)(kt & 1) != my_parity) {
-      // not this warp's stage
-    } else if (rows == GBK) {
-#pragma unroll
-      for (int kk = 0; kk < GBK / 4; ++kk) {
-        const int k = kk * 4 + q;
-        const T wv = w_base[k];
-        double a[8], b[4];
-#pragma unroll
-        for (int tp = 0; tp < 4; ++tp) {
-          const vec2 v = *reinterpret_cast<const vec2*>(a_base + k * PITCH + tp * 16);
-          a[2 * tp] = (double)Rn<T>::mul(v.x, wv);       // rn(w*x) in the model dtype == WX of the reference
-          a[2 * tp + 1] = (double)Rn<T>::mul(v.y, wv);
-        }
-#pragma unroll
-        for (int up = 0; up < 2; ++up) {
-          const vec2 v = *reinterpret_cast<const vec2*>(b_base + k * PITCH + up * 16);
-          b[2 * up] = (double)v.x;
-          b[2 * up + 1] = (double)v.y;
-        }
-#pragma unroll
-        for (int t = 0; t < 8; ++t)
-#pragma unroll
-          for (int u = 0; u < 4; ++u) dmma884(acc[t][u][0], acc[t][u][1], a[t], b[u]);
-      }
-    } else {
-      // tail stage: rows past the end of the unit were never copied - feed exact zeros instead
-#pragma unroll 1
-      for (int kk = 0; kk * 4 < rows; ++kk) {
-        const int k = kk * 4 + q;
-        const bool ok = k < rows;
-        const T wv = ok ? w_base[k] : T(0);
-        double a[8], b[4];
-#pragma unroll
-        for (int tp = 0; tp < 4; ++tp) {
-          vec2 v; v.x = T(0); v.y = T(0);
-          if (ok) v = *reinterpret_cast<const vec2*>(a_base + k * PITCH + tp * 16);
-          a[2 * tp] = ok ? (double)Rn<T>::mul(v.x, wv) : 0.0;
-          a[2 * tp + 1] = ok ? (double)Rn<T>::mul(v.y, wv) : 0.0;
-        }
-#pragma unroll
-        for (int up = 0; up < 2; ++up) {
-          vec2 v; v.x = T(0); v.y = T(0);
-          if (ok) v = *reinterpret_cast<const vec2*>(b_base + k * PITCH + up * 16);
-          b[2 * up] = (double)v.x;
-          b[2 * up + 1] = (double)v.y;
-        }
-#pragma unroll
-        for (int t = 0; t < 8; ++t)
-#pragma unroll
-          for (int u = 0; u < 4; ++u) dmma884(acc[t][u][0], acc[t][u][1], a[t], b[u]);
-      }
+  if (!diag) {
+    gram_rows<T, GBANDS_ALL>(acc, sA, sB, sW, full, empty, nrows, wm * 64, wn * 32);
+  } else {
+    // each warp's fixed band set, chosen once outside the row loop (the branch is warp-uniform)
+    const int src = warp == 4 ? GDIAG_OWNER4 : warp == 5 ? GDIAG_OWNER5 : warp;   // whose warp tile this warp computes
+    const int r0 = (src >> 2) * 64, c0 = (src & 3) * 32;
+    switch (warp) {
+      case 0: case 6: gram_rows<T, GDIAG_MASK[0]>(acc, sA, sA, sW, full, empty, nrows, r0, c0); break;
+      case 1: case 7: gram_rows<T, GDIAG_MASK[1]>(acc, sA, sA, sW, full, empty, nrows, r0, c0); break;
+      case 2: gram_rows<T, GDIAG_MASK[2]>(acc, sA, sA, sW, full, empty, nrows, r0, c0); break;
+      case 3: gram_rows<T, GDIAG_MASK[3]>(acc, sA, sA, sW, full, empty, nrows, r0, c0); break;
+      case 4: gram_rows<T, GDIAG_MASK[4]>(acc, sA, sA, sW, full, empty, nrows, r0, c0); break;
+      default: gram_rows<T, GDIAG_MASK[5]>(acc, sA, sA, sW, full, empty, nrows, r0, c0); break;
     }
-    __syncwarp();
-    if (lane == 0) mbar_arrive(empty + slot);
   }
   if (FUSE && fused_epi) {
     // The fold's mean / std rows are complete once the producer warps of every diagonal tile have signalled - and in a
     // diagonal tile this is also what says that ITS producer warps have read the last stages: the ring must not be reused
-    // (split-K merge, epilogue tile) before that.
+    // (band hand-over, epilogue tile) before that.
     if (tid == 0) {
       int seen;
       do {
@@ -489,30 +568,14 @@ __global__ void __launch_bounds__(GLAUNCH, 1) k_gram(const GramParams<T> p) {   
   compute_barrier();   // every stage consumed by every compute warp: the ring can be reused as the epilogue tile
 
   if (diag) {
-    // merge the helpers' partial accumulators into the owners' (warp 4 -> 6, warp 5 -> 7)
-    double* hbuf = reinterpret_cast<double*>(smem_raw);          // [2][GACC][32]
-    if (helper) {
-      double* dst = hbuf + (size_t)wn * GACC * 32 + lane;
-#pragma unroll
-      for (int t = 0; t < 8; ++t)
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          dst[((t * 4 + u) * 2 + 0) * 32] = acc[t][u][0];
-          dst[((t * 4 + u) * 2 + 1) * 32] = acc[t][u][1];
-          acc[t][u][0] = acc[t][u][1] = 0.0;                     // the helper's own tile is below the diagonal
-        }
-    }
+    // hand the bands computed for another warp's tile to their standard owners (warp 4 -> 3, warp 5 -> 2), so that every
+    // thread holds its own warp tile in the standard fragment layout, with zeros in the bands below the diagonal
+    double* hbuf = reinterpret_cast<double*>(smem_raw);          // [2][GACC][32]: slot 0 from warp 4, slot 1 from warp 5
+    if (warp == 4) gram_bands_out<GDIAG_MASK[4]>(acc, hbuf + lane);
+    if (warp == 5) gram_bands_out<GDIAG_MASK[5]>(acc, hbuf + (size_t)GACC * 32 + lane);
     compute_barrier();
-    if (half && !helper) {
-      const double* src = hbuf + (size_t)(wn - 2) * GACC * 32 + lane;
-#pragma unroll
-      for (int t = 0; t < 8; ++t)
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          acc[t][u][0] += src[((t * 4 + u) * 2 + 0) * 32];
-          acc[t][u][1] += src[((t * 4 + u) * 2 + 1) * 32];
-        }
-    }
+    if (warp == GDIAG_OWNER4) gram_bands_in<GDIAG_MASK[4]>(acc, hbuf + lane);
+    if (warp == GDIAG_OWNER5) gram_bands_in<GDIAG_MASK[5]>(acc, hbuf + (size_t)GACC * 32 + lane);
     compute_barrier();
   }
 
