@@ -67,6 +67,8 @@ SIGNATURES = {
     "cvmx_validation_rows": (_i32, [_vp, _i64, _vp, _u32, _vp, _vp, _i32]),
     "cvmx_pls_cv": (_i32, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i32]),
     "cvmx_ridge_cv": (_i32, [_vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _i32]),
+    "cvmx_pls_cv_predict": (_i32, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i32]),
+    "cvmx_ridge_cv_predict": (_i32, [_vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i32]),
     "cvmx_ridge_plan": (_i32, [_i64, _i64, _i64, _i64, _i32, _i32, _i32, _vp]),
     "cvmx_profile_enable": (_i32, [_vp, _i32]),
     "cvmx_profile_read": (_i32, [_vp, C.POINTER(_dbl), C.POINTER(_i64)]),

@@ -98,6 +98,8 @@ struct cvmx_handle {
   DevBuf pls_ws, pls_tab, pls_part, pls_out;
   // cross-validated ridge (cvmx_ridge_cv): pass scratch (cvmx_ridge_plan's layout), PRESS chunk table and partials, penalties
   DevBuf ridge_ws, ridge_tab, ridge_part, ridge_alpha;
+  // out-of-fold predictions of both for host outputs: one PRESS launch's rows, at most CV_PRED_STAGE_BYTES (one chunk's rows)
+  DevBuf cv_pred;
   // fused fit + folds (cvmx_fit_folds): raw float64 Gram of every fold of a true partition, [P][ntiles][GACC][GTHREADS],
   // valid while csr_version == fold_gram_version; cvmx_training_batch then only runs statistics + epilogue
   TableCache tc_gram, tc_finish;
@@ -1726,7 +1728,7 @@ int32_t training_impl(cvmx_t* h, const int64_t* d_off, const int64_t* d_idx, con
 // fold scalars in library scratch, the PLS kernels fit every fold, the PRESS kernels score its validation rows.
 template <typename T>
 int32_t pls_cv_impl(cvmx_t* h, int64_t f0, int64_t f1, int64_t A, void* opress, void* osumw, void* oB, int32_t* onfit,
-                    int32_t* ostatus, int32_t mem) {
+                    int32_t* ostatus, void* opred, int32_t mem) {
   const size_t sz = sizeof(T);
   const int64_t K = h->K, M = h->M;
   const uint32_t want = CVMX_WANT_XTX | CVMX_WANT_XTY;
@@ -1780,13 +1782,25 @@ int32_t pls_cv_impl(cvmx_t* h, int64_t f0, int64_t f1, int64_t A, void* opress, 
     CU(h, h->pls_part.reserve((size_t)std::max<int64_t>(nch, 1) * (A * M + 1) * sizeof(double)));
     double* part = h->pls_part.as<double>();
     double* part_w = part + nch * A * M;
-    if (nch > 0) {
+    // predictions: device outputs are written in place (row 0 of the window = CSR position off[c0]); host outputs are
+    // staged per launch, so PRESS then runs in launches of at most `per` chunks (partials land in the same slots)
+    const int64_t AM = A * M;
+    const int64_t per = opred && host ? std::max<int64_t>(1, CV_PRED_STAGE_BYTES / (PRESS_ROWS * AM * (int64_t)sz)) : std::max<int64_t>(nch, 1);
+    if (opred && host && nch > 0) CU(h, h->cv_pred.reserve((size_t)std::min(per, nch) * PRESS_ROWS * AM * sz));
+    for (int64_t g0 = 0; g0 < nch; g0 += per) {
+      const int64_t g1 = std::min(nch, g0 + per);
+      const int64_t p0 = tab[3 * g0], p1 = tab[3 * (g1 - 1)] + tab[3 * (g1 - 1) + 1];   // CSR positions of the launch
       PressParams<T> pp;
       pp.Z = h->Z.as<T>(); pp.w = h->weighted ? h->w.as<T>() : nullptr; pp.ld = h->ld;
-      pp.idx = h->d_idx.as<int64_t>(); pp.chunks = h->pls_tab.as<int64_t>(); pp.stats = h->stats.as<T>();
-      pp.flags = h->flags; pp.s = st; pp.part = part; pp.part_w = part_w;
-      k_pls_press<T><<<(unsigned)nch, PLS_THREADS, smem_press, h->stream>>>(pp);
+      pp.idx = h->d_idx.as<int64_t>(); pp.chunks = h->pls_tab.as<int64_t>() + 3 * g0; pp.stats = h->stats.as<T>();
+      pp.flags = h->flags; pp.s = st; pp.part = part + g0 * AM; pp.part_w = part_w + g0;
+      pp.pred = !opred ? nullptr : host ? h->cv_pred.as<T>() : (T*)opred + (off[c0] - off[f0]) * AM;
+      pp.pred_ld = AM;
+      pp.pred_pos = host ? p0 : off[c0];
+      k_pls_press<T><<<(unsigned)(g1 - g0), PLS_THREADS, smem_press, h->stream>>>(pp);
       h->launches++;
+      if (opred && host)
+        CU(h, cudaMemcpyAsync((T*)opred + (p0 - off[f0]) * AM, pp.pred, (size_t)(p1 - p0) * AM * sz, cudaMemcpyDeviceToHost, h->stream));
     }
     // outputs: straight into the caller's device buffers, or staged for the copy to the host
     T *dpress = (T*)opress + (size_t)d * A * M, *dsumw = (T*)osumw + d, *dB = oB ? (T*)oB + (size_t)d * A * K * M : nullptr;
@@ -1830,7 +1844,7 @@ int32_t pls_cv_impl(cvmx_t* h, int64_t f0, int64_t f1, int64_t A, void* opress, 
 // outputs of a pass are one contiguous range of the caller's arrays.
 template <typename T>
 int32_t ridge_cv_impl(cvmx_t* h, int64_t f0, int64_t f1, const double* alphas, int64_t L, void* opress, void* osumw, void* oB,
-                      int32_t* oinfo, int32_t* ostatus, int32_t mem, const int64_t* plan) {
+                      int32_t* oinfo, int32_t* ostatus, void* opred, int32_t mem, const int64_t* plan) {
   const size_t sz = sizeof(T);
   const int64_t K = h->K, M = h->M;
   const uint32_t want = CVMX_WANT_XTX | CVMX_WANT_XTY;
@@ -1852,6 +1866,11 @@ int32_t ridge_cv_impl(cvmx_t* h, int64_t f0, int64_t f1, const double* alphas, i
   CU(h, h->ridge_alpha.reserve((size_t)L * sizeof(double)));
   CU(h, h->out_xx.reserve((size_t)W * K * K * sz));
   CU(h, h->out_xy.reserve((size_t)W * K * M * sz));
+  // host predictions: a PRESS launch holds at most as many chunks as fill CV_PRED_STAGE_BYTES at the pass's width (and at
+  // most the plan's G), and never more rows than the range has; the bound below covers every pass width <= Lp M
+  const int64_t chunk_bytes = PRESS_ROWS * Lp * M * (int64_t)sz, range_bytes = (h->h_off[f1] - h->h_off[f0]) * Lp * M * (int64_t)sz;
+  if (opred && host && range_bytes > 0)
+    CU(h, h->cv_pred.reserve((size_t)std::min({G * chunk_bytes, std::max(CV_PRED_STAGE_BYTES, chunk_bytes), range_bytes})));
   // the penalties live on the device before any kernel runs; kernels never see a host address
   CU(h, cudaMemcpyAsync(h->ridge_alpha.p, alphas, (size_t)L * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   char* ws = h->ridge_ws.as<char>();
@@ -1914,20 +1933,34 @@ int32_t ridge_cv_impl(cvmx_t* h, int64_t f0, int64_t f1, const double* alphas, i
           h->launches++;
         }
       }
-      // PRESS over the window's chunks, at most G chunks per launch, each launch's sums added in chunk order
-      for (int64_t g0 = 0; g0 < nch; g0 += G) {
-        const int64_t g1 = std::min(nch, g0 + G);
+      // PRESS over the window's chunks, at most Gl chunks per launch, each launch's sums added in chunk order (the
+      // sums do not depend on the group size).  Predictions of the pass: columns [l0 M, l0 M + width) of rows [n][L M]
+      const int64_t Gl = opred && host ? std::min(G, std::max<int64_t>(1, CV_PRED_STAGE_BYTES / (PRESS_ROWS * width * (int64_t)sz))) : G;
+      for (int64_t g0 = 0; g0 < nch; g0 += Gl) {
+        const int64_t g1 = std::min(nch, g0 + Gl);
+        const int64_t p0 = tab[3 * g0], p1 = tab[3 * (g1 - 1)] + tab[3 * (g1 - 1) + 1];   // CSR positions of the launch
         RidgePressParams<T> pp;
         pp.Z = h->Z.as<T>(); pp.w = h->weighted ? h->w.as<T>() : nullptr; pp.ld = h->ld;
         pp.idx = h->d_idx.as<int64_t>(); pp.chunks = dtab + 3 * g0; pp.stats = h->stats.as<T>();
         pp.flags = h->flags; pp.s = st;
         pp.part = h->ridge_part.as<double>(); pp.part_w = pp.part + (g1 - g0) * width;
+        pp.pred = !opred ? nullptr : host ? h->cv_pred.as<T>() : (T*)opred + (off[c0] - off[f0]) * L * M + l0 * M;
+        pp.pred_ld = host ? width : L * M;
+        pp.pred_pos = host ? p0 : off[c0];
         const dim3 gp((unsigned)(g1 - g0), (unsigned)ridge_cdiv(width, RIDGE_PC));
         k_ridge_press<T><<<gp, RIDGE_THREADS, smem[CVMX_RK_PRESS], h->stream>>>(pp);
         const int64_t fa = tab[3 * g0 + 2], fb = tab[3 * (g1 - 1) + 2] + 1;
         k_ridge_press_accum<<<(unsigned)(fb - fa), RIDGE_THREADS, 0, h->stream>>>(pp.part, pp.part_w, dtab + 3 * nch, g0, g1, fa,
                                                                                   width, acc, acc_w);
         h->launches += 2;
+        if (opred && host) {
+          T* dst = (T*)opred + (p0 - off[f0]) * L * M + l0 * M;
+          if (width == L * M)
+            CU(h, cudaMemcpyAsync(dst, pp.pred, (size_t)(p1 - p0) * width * sz, cudaMemcpyDeviceToHost, h->stream));
+          else   // a one-fold pass over some of the penalties: a strided slice of the caller's rows
+            CU(h, cudaMemcpy2DAsync(dst, (size_t)L * M * sz, pp.pred, (size_t)width * sz, (size_t)width * sz, (size_t)(p1 - p0),
+                                    cudaMemcpyDeviceToHost, h->stream));
+        }
       }
       k_ridge_finish<T><<<(unsigned)Pn, RIDGE_THREADS, 0, h->stream>>>(st, acc, acc_w, dpress, dinfo, dsumw);
       h->launches++;
@@ -2071,7 +2104,7 @@ int32_t cvmx_destroy(cvmx_t* h) {
   for (DevBuf* b : {&h->stat_flags, &h->peer_sum, &h->w_glob, &h->g_off, &h->g_idx, &h->scan_look, &h->loo_ops, &h->Z, &h->w, &h->Ttot, &h->sum_z, &h->sumsq_z, &h->fit_scal, &h->d_off, &h->d_idx, &h->a_off, &h->a_idx,
                     &h->units, &h->tiles, &h->fold_units, &h->split_folds, &h->partials, &h->stats, &h->rawsums, &h->fscal, &h->pwcols,
                     &h->errflag, &h->out_xx, &h->out_xy, &h->out_small, &h->scan_seg, &h->scan_ok, &h->scan_list, &h->scan_cnt, &h->ystage, &h->fold_gram, &h->fold_raw, &h->chunk_ranges,
-                    &h->pls_ws, &h->pls_tab, &h->pls_part, &h->pls_out, &h->ridge_ws, &h->ridge_tab, &h->ridge_part, &h->ridge_alpha})
+                    &h->pls_ws, &h->pls_tab, &h->pls_part, &h->pls_out, &h->ridge_ws, &h->ridge_tab, &h->ridge_part, &h->ridge_alpha, &h->cv_pred})
     b->release();
   h->tc_gram.release(); h->tc_finish.release();
   delete h->stager; h->stager = nullptr;
@@ -2510,6 +2543,11 @@ int32_t cvmx_validation_rows(cvmx_t* h, int64_t fold, const void* stats, uint32_
 
 int32_t cvmx_pls_cv(cvmx_t* h, int64_t f0, int64_t f1, int64_t n_components, void* out_press, void* out_sum_w_val, void* out_B,
                     int32_t* out_n_fitted, int32_t* out_status, int32_t mem) {
+  return cvmx_pls_cv_predict(h, f0, f1, n_components, out_press, out_sum_w_val, out_B, out_n_fitted, out_status, nullptr, mem);
+}
+
+int32_t cvmx_pls_cv_predict(cvmx_t* h, int64_t f0, int64_t f1, int64_t n_components, void* out_press, void* out_sum_w_val,
+                            void* out_B, int32_t* out_n_fitted, int32_t* out_status, void* out_pred, int32_t mem) {
   if (!h || !h->fitted) return fail(h, CVMX_ERR_INVALID, "cvmx_pls_cv: fit first");
   if (h->slab) return fail(h, CVMX_ERR_INVALID, "cvmx_pls_cv: not available for a row-slab handle");
   if (f0 < 0 || f1 > h->P || f0 > f1) return fail(h, CVMX_ERR_INVALID, "cvmx_pls_cv: fold range outside the CSR");
@@ -2522,8 +2560,8 @@ int32_t cvmx_pls_cv(cvmx_t* h, int64_t f0, int64_t f1, int64_t n_components, voi
     return fail(h, CVMX_ERR_INVALID, "cvmx_pls_cv: an output pointer is NULL");
   ON_DEVICE(h);
   return h->dtype == CVMX_F64
-             ? pls_cv_impl<double>(h, f0, f1, n_components, out_press, out_sum_w_val, out_B, out_n_fitted, out_status, mem)
-             : pls_cv_impl<float>(h, f0, f1, n_components, out_press, out_sum_w_val, out_B, out_n_fitted, out_status, mem);
+             ? pls_cv_impl<double>(h, f0, f1, n_components, out_press, out_sum_w_val, out_B, out_n_fitted, out_status, out_pred, mem)
+             : pls_cv_impl<float>(h, f0, f1, n_components, out_press, out_sum_w_val, out_B, out_n_fitted, out_status, out_pred, mem);
 }
 
 int32_t cvmx_ridge_plan(int64_t K, int64_t M, int64_t L, int64_t P, int32_t dtype, int32_t mem, int32_t want_B, int64_t* plan) {
@@ -2534,6 +2572,12 @@ int32_t cvmx_ridge_plan(int64_t K, int64_t M, int64_t L, int64_t P, int32_t dtyp
 
 int32_t cvmx_ridge_cv(cvmx_t* h, int64_t f0, int64_t f1, const double* alphas, int64_t L, void* out_press, void* out_sum_w_val,
                       void* out_B, int32_t* out_info, int32_t* out_status, int32_t mem) {
+  return cvmx_ridge_cv_predict(h, f0, f1, alphas, L, out_press, out_sum_w_val, out_B, out_info, out_status, nullptr, mem);
+}
+
+int32_t cvmx_ridge_cv_predict(cvmx_t* h, int64_t f0, int64_t f1, const double* alphas, int64_t L, void* out_press,
+                              void* out_sum_w_val, void* out_B, int32_t* out_info, int32_t* out_status, void* out_pred,
+                              int32_t mem) {
   if (!h || !h->fitted) return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: fit first");
   if (h->slab) return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: not available for a row-slab handle");
   if (f0 < 0 || f1 > h->P || f0 > f1) return fail(h, CVMX_ERR_INVALID, "cvmx_ridge_cv: fold range outside the CSR");
@@ -2554,8 +2598,8 @@ int32_t cvmx_ridge_cv(cvmx_t* h, int64_t f0, int64_t f1, const double* alphas, i
                                          " cannot run within the device limits");
   ON_DEVICE(h);
   return h->dtype == CVMX_F64
-             ? ridge_cv_impl<double>(h, f0, f1, alphas, L, out_press, out_sum_w_val, out_B, out_info, out_status, mem, plan)
-             : ridge_cv_impl<float>(h, f0, f1, alphas, L, out_press, out_sum_w_val, out_B, out_info, out_status, mem, plan);
+             ? ridge_cv_impl<double>(h, f0, f1, alphas, L, out_press, out_sum_w_val, out_B, out_info, out_status, out_pred, mem, plan)
+             : ridge_cv_impl<float>(h, f0, f1, alphas, L, out_press, out_sum_w_val, out_B, out_info, out_status, out_pred, mem, plan);
 }
 
 int32_t cvmx_profile_enable(cvmx_t* h, int32_t on) {

@@ -25,6 +25,9 @@ constexpr int PLS_ROWS_PER_BLOCK = PLS_WARPS;   // k_pls_xtx_r: one warp per row
 constexpr int PRESS_ROWS = 32;    // validation rows per PRESS chunk (a chunk never spans two folds)
 constexpr int PRESS_AT = 64;      // components per tile of t = x~ R^T
 constexpr int PRESS_KT = 32;      // columns per tile
+// out-of-fold predictions for HOST outputs: the rows of one PRESS launch are staged in one device buffer of at most this
+// many bytes (or one chunk's rows when a chunk alone is larger) and copied out before the buffer is reused
+constexpr int64_t CV_PRED_STAGE_BYTES = (int64_t)256 << 20;
 
 enum { PLS_ACTIVE = 0, PLS_STOPPED = 1, PLS_BAD = 2 };
 
@@ -286,6 +289,8 @@ __global__ void __launch_bounds__(PLS_THREADS) k_pls_coefs(PlsState s, T* __rest
 // PRESS of one chunk of at most PRESS_ROWS validation rows of one fold.  chunks[c] = {first CSR position, rows, fold}.
 // Per row: x~ = (x - mu_X) / sigma_X (as the flags say), t = x~ R^T, y^(a) = sum_{j <= a} t_j q_j^T, prediction
 // y^(a) * sigma_Y + mu_Y; part[c][a][m] = sum over the chunk's rows (in row order) of w (y - prediction)^2.
+// With pred set, the thread that forms a prediction also stores it (rounded once to T): CSR position q goes to row
+// q - pred_pos of pred, element a M + m; a refused fold's rows are NaN.
 template <typename T>
 struct PressParams {
   const T* Z; const T* w; int64_t ld;
@@ -296,6 +301,9 @@ struct PressParams {
   PlsState s;
   double* part;                    // [nchunks][A][M]
   double* part_w;                  // [nchunks]
+  T* pred;                         // [rows][pred_ld] device predictions, or nullptr: none stored
+  int64_t pred_ld;                 // row pitch of pred in elements (>= A M)
+  int64_t pred_pos;                // CSR position of pred's row 0
 };
 
 inline size_t press_smem_bytes(int64_t M) {
@@ -334,7 +342,16 @@ __global__ void __launch_bounds__(PLS_THREADS) k_pls_press(PressParams<T> p) {
   }
   const int state = p.s.state[f];
   double* out = p.part + c * A * M;
-  if (state == PLS_BAD) return;   // the reduce kernel writes NaN; the statistics of such a fold are not used
+  if (state == PLS_BAD) {   // the reduce kernel writes NaN press; the statistics of such a fold are not used
+    if (p.pred) {
+      const int64_t AM = A * M;
+      for (int64_t e = tid; e < n * AM; e += PLS_THREADS) {
+        const int64_t i = e / AM;
+        p.pred[(pos + i - p.pred_pos) * p.pred_ld + (e - i * AM)] = (T)__longlong_as_double(0x7ff8000000000000LL);
+      }
+    }
+    return;
+  }
   for (int64_t e = tid; e < PRESS_ROWS * M; e += PLS_THREADS) {
     const int64_t i = e / M, m = e - i * M;
     ys[e] = rows[i] < 0 ? 0.0 : (double)p.Z[rows[i] * ld + K + m];
@@ -384,6 +401,7 @@ __global__ void __launch_bounds__(PLS_THREADS) k_pls_press(PressParams<T> p) {
       const int64_t m = tid;
       const double mu = cY ? (double)mean[K + m] : 0.0, sd = sY ? (double)sdev[K + m] : 1.0;
       const int64_t a1 = A - a0 < PRESS_AT ? A - a0 : PRESS_AT;
+      T* prow = p.pred ? p.pred + (pos - p.pred_pos) * p.pred_ld + m : nullptr;   // row 0 of the chunk, column m
       for (int64_t j = 0; j < a1; ++j) {
         const int64_t aa = a0 + j;
         const double qm = aa < nf ? Q[aa * M + m] : 0.0;
@@ -395,6 +413,7 @@ __global__ void __launch_bounds__(PLS_THREADS) k_pls_press(PressParams<T> p) {
           double pred = y;
           if (sY) pred *= sd;
           if (cY) pred += mu;
+          if (prow) prow[i * p.pred_ld + aa * M] = (T)pred;
           const double res = ys[i * M + m] - pred;
           ss = fma(wv[i] * res, res, ss);
         }

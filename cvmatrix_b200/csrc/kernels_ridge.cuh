@@ -378,6 +378,8 @@ __global__ void __launch_bounds__(RIDGE_THREADS) k_ridge_bsolve_update(RidgeStat
 // col = l M + m.  chunks[c] = {first CSR position, rows, fold in window}.  Per row and column: x~ = (x - mu_X) /
 // sigma_X (as the flags say), prediction (x~ . b) * sigma_Y + mu_Y; part[c][col] = sum over the chunk's rows (in row
 // order) of w (y - prediction)^2, 0 for failed pairs and refused folds.  grid (chunks of the launch, column tiles).
+// With pred set, the thread that forms a prediction also stores it (rounded once to T): CSR position q goes to row
+// q - pred_pos of pred, element col; failed pairs and refused folds store NaN.
 template <typename T>
 struct RidgePressParams {
   const T* Z; const T* w; int64_t ld;
@@ -388,6 +390,9 @@ struct RidgePressParams {
   RidgeState s;
   double* part;                    // [nchunks][Lp M]
   double* part_w;                  // [nchunks]
+  T* pred;                         // [rows][pred_ld] device predictions from the pass's column 0, or nullptr: none stored
+  int64_t pred_ld;                 // row pitch of pred in elements (>= Lp M)
+  int64_t pred_pos;                // CSR position of pred's row 0
 };
 
 template <typename T>
@@ -430,7 +435,13 @@ __global__ void __launch_bounds__(RIDGE_THREADS) k_ridge_press(RidgePressParams<
   bool any = false;
   for (int i = 0; i < RIDGE_PC; ++i) any |= cbase[i] >= 0;
   if (!any) {   // refused fold or only failed pairs: nothing below touches the statistics or the matrices
-    if (tid < RIDGE_PC && col0 + tid < width) p.part[c * width + col0 + tid] = 0.0;
+    if (tid < RIDGE_PC && col0 + tid < width) {
+      p.part[c * width + col0 + tid] = 0.0;
+      if (p.pred) {
+        T* pc = p.pred + (pos - p.pred_pos) * p.pred_ld + col0 + tid;
+        for (int i = 0; i < n; ++i) pc[i * p.pred_ld] = (T)__longlong_as_double(0x7ff8000000000000LL);
+      }
+    }
     return;
   }
   const int trow = tid / 8, tc = tid % 8;   // thread owns row trow, columns tc + 8 i
@@ -468,6 +479,7 @@ __global__ void __launch_bounds__(RIDGE_THREADS) k_ridge_press(RidgePressParams<
   __syncthreads();
   if (tid < RIDGE_PC && col0 + tid < width) {
     const int64_t col = col0 + tid, m = col % M;
+    T* pc = p.pred ? p.pred + (pos - p.pred_pos) * p.pred_ld + col : nullptr;   // row 0 of the chunk, column col
     double ss = 0.0;
     if (cbase[tid] >= 0) {
       const double mu = cY ? (double)mean[K + m] : 0.0, sd = sY ? (double)sdev[K + m] : 1.0;
@@ -475,9 +487,12 @@ __global__ void __launch_bounds__(RIDGE_THREADS) k_ridge_press(RidgePressParams<
         double pred = ps[i * RIDGE_PC + tid];
         if (sY) pred *= sd;
         if (cY) pred += mu;
+        if (pc) pc[i * p.pred_ld] = (T)pred;
         const double res = (double)p.Z[rows[i] * ld + K + m] - pred;
         ss = fma(wv[i] * res, res, ss);
       }
+    } else if (pc) {
+      for (int i = 0; i < n; ++i) pc[i * p.pred_ld] = (T)__longlong_as_double(0x7ff8000000000000LL);
     }
     p.part[c * width + col] = ss;
   }

@@ -550,7 +550,8 @@ class CVMatrix:
                 self._lib.cvmx_sync(self._h)
 
     def pls_cross_validate(self, n_components: int, fold_begin: int = 0, fold_end: Optional[int] = None,
-                           return_coefs: bool = False, out: str = "numpy", check: bool = True):
+                           return_coefs: bool = False, out: str = "numpy", check: bool = True,
+                           return_predictions: bool = False):
         """
         Cross-validated PLS regression over folds ``[fold_begin, fold_end)`` of the CSR (see ``set_folds``), on the GPU.
 
@@ -567,11 +568,23 @@ class CVMatrix:
         errors of ``training_XTX_XTY`` are raised; without it such folds get NaN ``press`` / ``B`` and ``n_fitted`` 0.
         A ``UserWarning`` names folds that stopped early.
 
+        With ``return_predictions`` the dict also holds the out-of-fold predictions the PRESS is formed from:
+        ``predictions`` (n, A, M), row j the prediction of the j-th validation index of the range in CSR order (n = the
+        number of stored indices of folds ``[fold_begin, fold_end)``, repeats kept) with 1 .. A components, and ``rows``
+        (n,) int64, the data-set row of each (indices normalised to ``[0, N)``); without it the dict has neither key.
+        A refused fold's rows are NaN; a fold that stopped early repeats its last fitted component's predictions.
+
         Example - root mean squared error of cross-validation per number of components and response::
 
             cvm.fit(X, Y); cvm.set_folds(Partitioner(folds))
             r = cvm.pls_cross_validate(20)
             rmsecv = np.sqrt(r["press"].sum(0) / r["sum_w_val"].sum())    # (20, M)
+
+        Example - scikit-learn's ``cross_val_predict`` for every number of components (a ``Partitioner`` covers each
+        row once)::
+
+            r = cvm.pls_cross_validate(20, return_predictions=True)
+            Yhat = np.empty((N, 20, M)); Yhat[r["rows"]] = r["predictions"]
         """
         self._require_fit()
         if fold_end is None:
@@ -584,6 +597,7 @@ class CVMatrix:
         if M > 128:
             raise ValueError(f"at most 128 response columns are supported; Y has {M}")
         P = max(int(fold_end) - int(fold_begin), 0)
+        n_pred = self._prediction_count(fold_begin, fold_end)
         if out == "torch":
             import torch
 
@@ -594,6 +608,7 @@ class CVMatrix:
             n_fitted = torch.empty((P,), dtype=torch.int32, device=dev)
             status = torch.empty((P,), dtype=torch.int32, device=dev)
             B = torch.empty((P, A, K, M), dtype=tdt, device=dev) if return_coefs else None
+            pred = torch.empty((n_pred, A, M), dtype=tdt, device=dev) if return_predictions else None
             p, mem = _tptr, _lib.DEVICE
         elif out == "numpy":
             press = np.empty((P, A, M), dt)
@@ -601,12 +616,13 @@ class CVMatrix:
             n_fitted = np.zeros((P,), np.int32)
             status = np.zeros((P,), np.int32)
             B = np.empty((P, A, K, M), dt) if return_coefs else None
+            pred = np.empty((n_pred, A, M), dt) if return_predictions else None
             p, mem = _ptr, _lib.HOST
         else:
             raise ValueError("out must be 'numpy' or 'torch'")
         with self._torch_stream() if out == "torch" else contextlib.nullcontext():
-            rc = self._lib.cvmx_pls_cv(self._h, int(fold_begin), int(fold_end), A, p(press), p(sum_w), p(B), p(n_fitted),
-                                       p(status), mem)
+            rc = self._lib.cvmx_pls_cv_predict(self._h, int(fold_begin), int(fold_end), A, p(press), p(sum_w), p(B),
+                                               p(n_fitted), p(status), p(pred), mem)
             _lib.check(rc, self._h)
         st = status.cpu().numpy() if out == "torch" else status
         if check:
@@ -622,10 +638,13 @@ class CVMatrix:
             warnings.warn(f"{early.size} fold(s) stopped before {A} components (first: fold {int(fold_begin) + int(early[0])} "
                           f"with {int(nf[early[0]])}): the remaining XTY vanished; their later coefficients repeat the last ones",
                           UserWarning, stacklevel=2)
-        return dict(press=press, sum_w_val=sum_w, n_fitted=n_fitted, status=status, B=B)
+        r = dict(press=press, sum_w_val=sum_w, n_fitted=n_fitted, status=status, B=B)
+        if return_predictions:
+            r.update(predictions=pred, rows=self._prediction_rows(fold_begin, fold_end, out))
+        return r
 
     def ridge_cross_validate(self, alphas, fold_begin: int = 0, fold_end: Optional[int] = None, return_coefs: bool = False,
-                             out: str = "numpy", check: bool = True):
+                             out: str = "numpy", check: bool = True, return_predictions: bool = False):
         """
         Cross-validated ridge regression over folds ``[fold_begin, fold_end)`` of the CSR (see ``set_folds``) for every
         penalty in ``alphas``, on the GPU.
@@ -647,11 +666,22 @@ class CVMatrix:
         degenerate fold errors of ``training_XTX_XTY`` are raised; without it such folds get NaN ``press`` / ``B`` for
         every penalty and ``info`` 0.
 
+        With ``return_predictions`` the dict also holds the out-of-fold predictions the PRESS is formed from:
+        ``predictions`` (n, L, M), row j the prediction of the j-th validation index of the range in CSR order (n = the
+        number of stored indices of folds ``[fold_begin, fold_end)``, repeats kept) for every penalty, and ``rows``
+        (n,) int64, the data-set row of each (indices normalised to ``[0, N)``); without it the dict has neither key.
+        A refused fold's rows are NaN, and a pair with ``info != 0`` is NaN for that penalty only.
+
         Example - root mean squared error of cross-validation per penalty and response::
 
             cvm.fit(X, Y); cvm.set_folds(Partitioner(folds))
             r = cvm.ridge_cross_validate(np.logspace(-3, 3, 20))
             rmsecv = np.sqrt(r["press"].sum(0) / r["sum_w_val"].sum())    # (L, M)
+
+        Example - scikit-learn's ``cross_val_predict`` for every penalty (a ``Partitioner`` covers each row once)::
+
+            r = cvm.ridge_cross_validate(np.logspace(-3, 3, 20), return_predictions=True)
+            Yhat = np.empty((N, 20, M)); Yhat[r["rows"]] = r["predictions"]
         """
         self._require_fit()
         if fold_end is None:
@@ -672,6 +702,7 @@ class CVMatrix:
         if M > 128:
             raise ValueError(f"at most 128 response columns are supported; Y has {M}")
         P = max(int(fold_end) - int(fold_begin), 0)
+        n_pred = self._prediction_count(fold_begin, fold_end)
         if out == "torch":
             import torch
 
@@ -682,6 +713,7 @@ class CVMatrix:
             info = torch.empty((P, L), dtype=torch.int32, device=dev)
             status = torch.empty((P,), dtype=torch.int32, device=dev)
             B = torch.empty((P, L, K, M), dtype=tdt, device=dev) if return_coefs else None
+            pred = torch.empty((n_pred, L, M), dtype=tdt, device=dev) if return_predictions else None
             p, mem = _tptr, _lib.DEVICE
         elif out == "numpy":
             press = np.empty((P, L, M), dt)
@@ -689,12 +721,13 @@ class CVMatrix:
             info = np.zeros((P, L), np.int32)
             status = np.zeros((P,), np.int32)
             B = np.empty((P, L, K, M), dt) if return_coefs else None
+            pred = np.empty((n_pred, L, M), dt) if return_predictions else None
             p, mem = _ptr, _lib.HOST
         else:
             raise ValueError("out must be 'numpy' or 'torch'")
         with self._torch_stream() if out == "torch" else contextlib.nullcontext():
-            rc = self._lib.cvmx_ridge_cv(self._h, int(fold_begin), int(fold_end), _ptr(lam), L, p(press), p(sum_w), p(B),
-                                         p(info), p(status), mem)
+            rc = self._lib.cvmx_ridge_cv_predict(self._h, int(fold_begin), int(fold_end), _ptr(lam), L, p(press), p(sum_w),
+                                                 p(B), p(info), p(status), p(pred), mem)
             _lib.check(rc, self._h)
         if check:
             st = status.cpu().numpy() if out == "torch" else status
@@ -710,7 +743,28 @@ class CVMatrix:
             warnings.warn(f"{len(failed)} (fold, penalty) pair(s) could not be factored: XTX + alpha I is not positive "
                           f"definite (first: fold {int(fold_begin) + f}, alpha {lam[l]!r} at index {l}, pivot {int(inf[f, l])}); "
                           "their press and B are NaN", UserWarning, stacklevel=2)
-        return dict(press=press, sum_w_val=sum_w, info=info, status=status, B=B)
+        r = dict(press=press, sum_w_val=sum_w, info=info, status=status, B=B)
+        if return_predictions:
+            r.update(predictions=pred, rows=self._prediction_rows(fold_begin, fold_end, out))
+        return r
+
+    def _prediction_count(self, fold_begin, fold_end) -> int:
+        """Number of out-of-fold predictions of folds [fold_begin, fold_end): their stored CSR indices."""
+        f0, f1 = int(fold_begin), int(fold_end)
+        if not 0 <= f0 <= f1 <= getattr(self, "_n_folds", 0):
+            return 0    # the library reports the bad range
+        return int(self._offsets[f1] - self._offsets[f0])
+
+    def _prediction_rows(self, fold_begin, fold_end, out):
+        """Data-set row of every out-of-fold prediction of folds [fold_begin, fold_end): the CSR indices, normalised."""
+        idx = np.asarray(self._fold_indices[self._offsets[int(fold_begin)]:self._offsets[int(fold_end)]], np.int64)
+        neg = idx.size > 0 and idx.min() < 0
+        if out == "torch":
+            import torch
+
+            rows = torch.from_numpy(idx).to(torch.device("cuda", self.device))
+            return torch.where(rows < 0, rows + self.N, rows) if neg else rows
+        return np.where(idx < 0, idx + self.N, idx) if neg else idx.copy()
 
     def validation_rows(self, fold: int, stats: Optional[Stats] = None, out: str = "numpy"):
         """

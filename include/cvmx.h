@@ -316,6 +316,26 @@ int32_t cvmx_pls_cv(cvmx_t* h, int64_t fold_begin, int64_t fold_end, int64_t n_c
 int32_t cvmx_ridge_cv(cvmx_t* h, int64_t fold_begin, int64_t fold_end, const double* alphas, int64_t L, void* out_press,
                       void* out_sum_w_val, void* out_B, int32_t* out_info, int32_t* out_status, int32_t mem);
 
+/*
+ * cvmx_pls_cv / cvmx_ridge_cv that also return the out-of-fold predictions (cvmx_pls_cv and cvmx_ridge_cv are these
+ * calls with out_pred = NULL; every other output is bit-identical with and without predictions).  The predictions are
+ * in CSR order over the call's fold range: with off the CSR offsets and n = off[fold_end] - off[fold_begin], row j
+ * belongs to CSR entry off[fold_begin] + j (repeats kept as stored), in the handle's dtype (float32: rounded once from
+ * the float64 value), `mem` like the other outputs:
+ *   PLS    out_pred [n, A, M]  row j, component a: the prediction with a + 1 components whose residual PRESS adds,
+ *                              ((x - mu_X) / sigma_X) B_a * sigma_Y + mu_Y; a fold that stopped early repeats its last
+ *                              fitted component's predictions; n_fitted = 0 predicts mu_Y if centred, else 0
+ *   ridge  out_pred [n, L, M]  the same for penalty l; NaN for a pair with info != 0
+ * Rows of a fold refused by its status bits are NaN; empty folds have no rows.  out_pred may be NULL.  Host outputs are
+ * staged through at most 256 MiB of device memory per PRESS launch, or one 32-row chunk's predictions if that is larger.
+ */
+int32_t cvmx_pls_cv_predict(cvmx_t* h, int64_t fold_begin, int64_t fold_end, int64_t n_components, void* out_press,
+                            void* out_sum_w_val, void* out_B, int32_t* out_n_fitted, int32_t* out_status,
+                            void* out_pred, int32_t mem);
+int32_t cvmx_ridge_cv_predict(cvmx_t* h, int64_t fold_begin, int64_t fold_end, const double* alphas, int64_t L,
+                              void* out_press, void* out_sum_w_val, void* out_B, int32_t* out_info, int32_t* out_status,
+                              void* out_pred, int32_t mem);
+
 /* Host-only (no CUDA call): the launch plan cvmx_ridge_cv uses for K columns of X, M of Y, L penalties and P folds of
  * the given dtype, output memory (`mem`) and whether B is wanted.  plan[CVMX_RIDGE_PLAN_LEN] receives the folds per
  * window, the penalties per pass, the device scratch bytes of a pass and the byte offset at which each of its arrays

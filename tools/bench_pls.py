@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Cross-validated PLS on the GPU (CVMatrix.pls_cross_validate) against the fold path it builds on.
 
-    python tools/bench_pls.py --out DIR [--cases cfg2,cfg3,cfg4,cfg5s] [--reps 3] [--components 20]
+    python tools/bench_pls.py --out DIR [--cases cfg2,cfg3,cfg4,cfg5s] [--reps 3] [--components 20] [--predictions]
 
 Per case: inputs are generated on the device (uniform [0, 1), seed 42, weighted) and fitted through fit_begin /
 fit_rows / fit_end, the folds are arange(N) % P.  Timed with CUDA events on the same range and resident inputs:
@@ -11,7 +11,9 @@ run under torch.profiler gives the time of every kernel.  Bytes follow DESIGN.md
 for the XTX r products plus one read of the validation rows (K + M values each) for PRESS; the share of the HBM bound
 is (bytes / 7.7 TB/s) over the PLS + PRESS time.  The CPU figure is the numpy oracle (oracle/pls_oracle.py) timed on
 the engine's own matrices and validation rows for the first `cpu_folds` folds of the case, reported as such.
-Writes DIR/bench_pls.json (and one line per case to stdout).
+With --predictions the same call is also timed with ``return_predictions=True`` (out="torch"), alternating with the
+plain call in one loop, and the difference is reported beside the HBM bound of writing n * A * M * sizeof(T) bytes of
+predictions (n = N: the folds partition the rows).  Writes DIR/bench_pls.json (and one line per case to stdout).
 
 Cases (A = 20 components, float64, center + scale X and Y):
   cfg2   N = 1,000,000  K = 500   M = 10   P = 5
@@ -89,6 +91,32 @@ def timed(fn, reps):
     return ts
 
 
+def predictions_overhead(plain, with_pred, reps, pred_bytes):
+    """Median CUDA-event times of `plain` and `with_pred`, alternated in one loop after a warm-up of each, their
+    difference, and the HBM bound of writing the predictions."""
+    plain(), with_pred()
+    tp, tw = [], []
+    for _ in range(reps):
+        tp += timed_once(plain)
+        tw += timed_once(with_pred)
+    d = float(np.median(tw) - np.median(tp))
+    return dict(plain_ms=tp, with_predictions_ms=tw, overhead_ms=d,
+                overhead_share=d / float(np.median(tp)), prediction_bytes=pred_bytes,
+                prediction_write_hbm_bound_ms=pred_bytes / HBM_BPS * 1e3)
+
+
+def timed_once(fn):
+    import torch
+
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    torch.cuda.synchronize()
+    e0.record()
+    fn()
+    e1.record()
+    torch.cuda.synchronize()
+    return [e0.elapsed_time(e1)]
+
+
 def kernel_times(fn):
     import torch
     from torch.profiler import ProfilerActivity, profile
@@ -119,7 +147,7 @@ def cpu_oracle(m, A, n):
     return (time.perf_counter() - t0) * 1e3
 
 
-def run_case(name, A, reps):
+def run_case(name, A, reps, predictions=False):
     import torch
 
     c = CASES[name]
@@ -153,6 +181,10 @@ def run_case(name, A, reps):
                     "what": "oracle/pls_oracle.py IKPLS + PRESS on the engine's XTX / XTY / statistics / validation rows, "
                             "first folds only, host numpy"},
     )
+    if predictions:
+        pred = lambda: m.pls_cross_validate(A, out="torch", check=False, return_predictions=True)  # noqa: E731
+        out["predictions"] = predictions_overhead(pls, pred, reps, N * A * M * 8)
+        out["predictions"]["kernels"] = kernel_times(pred)
     del m
     torch.cuda.empty_cache()
     return out
@@ -164,6 +196,7 @@ def main():
     ap.add_argument("--cases", default="cfg2,cfg3,cfg4,cfg5s")
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--components", type=int, default=20)
+    ap.add_argument("--predictions", action="store_true", help="also time return_predictions=True against the plain call")
     a = ap.parse_args()
     import torch
 
@@ -172,9 +205,9 @@ def main():
     os.makedirs(a.out, exist_ok=True)
     res = {"device": device_info(), "cases": []}
     for name in a.cases.split(","):
-        r = run_case(name, a.components, a.reps)
+        r = run_case(name, a.components, a.reps, a.predictions)
         res["cases"].append(r)
-        print(json.dumps({k: v for k, v in r.items() if k != "kernels"}), flush=True)
+        print(json.dumps({k: v for k, v in r.items() if k != "kernels"}, default=str), flush=True)
     res["device_after"] = device_info()
     with open(os.path.join(a.out, "bench_pls.json"), "w") as f:
         json.dump(res, f, indent=1)

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Cross-validated ridge regression on the GPU (CVMatrix.ridge_cross_validate) against the fold path it builds on.
 
-    python tools/bench_ridge.py --out DIR [--cases cfg2,cfg3,cfg4,cfg5s] [--reps 3] [--penalties 20]
+    python tools/bench_ridge.py --out DIR [--cases cfg2,cfg3,cfg4,cfg5s] [--reps 3] [--penalties 20] [--predictions]
 
 Per case: inputs are generated on the device (uniform [0, 1), seed 42, weighted) and fitted through fit_begin /
 fit_rows / fit_end, the folds are arange(N) % P, the penalties are L log-spaced values over 1e-3 .. 1e3 times
@@ -11,7 +11,9 @@ out="torch")`` (the same matrices into library scratch, then the factorisations,
 difference is the cost of ridge + PRESS.  A separate run under torch.profiler gives the time of every kernel.  The flop
 model counts P L K^3 / 3 for the factorisations, 2 P L K^2 M for the substitutions and 2 n_val K L M for PRESS; the
 achieved FP64 rate of the factorisation is its flops over the summed time of k_ridge_potrf_diag, k_ridge_trsm and
-k_ridge_syrk.  The device name and power limit are read in the same run.  Writes DIR/bench_ridge.json (and one line
+k_ridge_syrk.  The device name and power limit are read in the same run.  With --predictions the same call is also
+timed with ``return_predictions=True`` (out="torch"), alternating with the plain call, and the difference is reported
+beside the HBM bound of writing n * L * M * sizeof(T) bytes of predictions.  Writes DIR/bench_ridge.json (and one line
 per case to stdout).
 
 Cases (float64, center + scale X and Y):
@@ -34,7 +36,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 
-from bench_pls import CASES, device_info, make_model, timed  # noqa: E402
+from bench_pls import CASES, device_info, make_model, predictions_overhead, timed  # noqa: E402
 
 FACTOR_KERNELS = ("k_ridge_potrf_diag", "k_ridge_trsm", "k_ridge_syrk")
 
@@ -60,7 +62,7 @@ def flop_model(N, K, M, P, L):
     return {"factorisation": P * L * K**3 / 3, "substitutions": 2 * P * L * K**2 * M, "press": 2 * N * K * L * M}
 
 
-def run_case(name, L, reps):
+def run_case(name, L, reps, predictions=False):
     import torch
 
     c = CASES[name]
@@ -91,7 +93,12 @@ def run_case(name, L, reps):
         failed_pairs=n_failed,
         best_penalty_index=[int(i) for i in np.argmin(rmsecv, axis=0)[:3]],
     )
-    del m, r
+    del r
+    if predictions:
+        pred = lambda: m.ridge_cross_validate(alphas, out="torch", check=False, return_predictions=True)  # noqa: E731
+        out["predictions"] = predictions_overhead(ridge, pred, reps, N * L * M * 8)
+        out["predictions"]["kernels"] = kernel_times(pred)
+    del m
     torch.cuda.empty_cache()
     return out
 
@@ -102,6 +109,7 @@ def main():
     ap.add_argument("--cases", default="cfg2,cfg3,cfg4,cfg5s")
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--penalties", type=int, default=20)
+    ap.add_argument("--predictions", action="store_true", help="also time return_predictions=True against the plain call")
     a = ap.parse_args()
     import torch
 
@@ -110,7 +118,7 @@ def main():
     os.makedirs(a.out, exist_ok=True)
     res = {"device": device_info(), "cases": []}
     for name in a.cases.split(","):
-        r = run_case(name, a.penalties, a.reps)
+        r = run_case(name, a.penalties, a.reps, a.predictions)
         res["cases"].append(r)
         print(json.dumps({k: v for k, v in r.items() if k != "kernels"}), flush=True)
     res["device_after"] = device_info()
